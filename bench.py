@@ -17,6 +17,7 @@ GT-only, ~4.3 GB) — each tool makes its own full pass, exactly like the two re
   cli       wall clock of the drop-in executables on the 4.3 GB file (page cache), reference tools beside them
   --impl reference : the unmodified reference tools (oracle/_ref/VCFX_*, built by oracle/Makefile from the
             reference sources) on this box's host cores, each step on a bounded sample of the same workload
+  --dump-outputs DIR : what the timed job computed in its last step, as DIR/<name>.npy (float32 / float64)
 
 N > 1 (torchrun, one rank per GPU): every rank owns its own newline-aligned shard of the same synthetic
 stream (weak scaling, no data-path collective); the scalar totals cross ranks in one tiny NCCL all-reduce
@@ -233,7 +234,7 @@ def run_reference_arm(args):
     warm = max(0, min(args.warmup, 1))        # one warm-up run is enough for a process that streams a cached file
     r = cpu_reference_run(CPU_SAMPLE_VARIANTS, args.steps, warm)
     if r is None:
-        print(json.dumps({"impl": "reference", "unavailable": "oracle/_ref/VCFX_* not built (run make -C oracle ref where /root/reference exists)"}))
+        print(json.dumps({"impl": "reference", "unavailable": "oracle/_ref/VCFX_* not built (make -C oracle ref REFERENCE=<VCFX source tree>)"}))
         return 0
     ms = 1e3 * sum(r["times"]) / len(r["times"])
     sample = (f"{r['variants']} variants x {SAMPLES} samples ({r['bytes'] / 1e9:.2f} GB): a prefix of the C2 stream, file in page cache; "
@@ -252,6 +253,29 @@ def run_reference_arm(args):
     }
     print(json.dumps(line))
     return 0
+
+
+DUMP_SAMPLE_ROWS = 4096
+
+
+def dump_outputs(np, out_dir: Path, suffix: str, af_text: bytes, af_rows: int, vc_rows: int):
+    """What one step of the timed job hands its caller, as float arrays (DIR/<name><suffix>.npy), so that two builds
+    can be compared output for output: POS and allele frequency of every allele_freq_calc row, the text of a fixed,
+    seeded sample of its rows as byte values, and the row counts of both tools."""
+    rows = af_text.splitlines(keepends=True)
+    assert len(rows) == af_rows, (len(rows), af_rows)
+    cols = [r.split(b"\t") for r in rows]
+    pick = np.sort(np.random.default_rng(0).choice(len(rows), min(DUMP_SAMPLE_ROWS, len(rows)), replace=False))
+    arrays = {
+        "allele_freq_calc_pos": np.array([float(c[1]) for c in cols], dtype=np.float64),
+        "allele_freq_calc_af": np.array([float(c[-1]) for c in cols], dtype=np.float64),
+        "allele_freq_calc_text_sample": np.frombuffer(b"".join(rows[i] for i in pick), dtype=np.uint8).astype(np.float32),
+        "row_counts": np.array([af_rows, vc_rows], dtype=np.float64),
+    }
+    out_dir.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(out_dir / f"{name}{suffix}.npy", a)
+    log(f"[bench] wrote {', '.join(f'{n}{suffix}.npy' for n in arrays)} to {out_dir} ({sum(a.nbytes for a in arrays.values()) / 1e6:.1f} MB)")
 
 
 def workload_config():
@@ -630,7 +654,8 @@ def hwe_pvalue_report(api, O, np):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10,
+                    help="timed steps of the headline (resident) and e2e legs; the per-kernel medians and the configs entries use fixed counts")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="vcfx_b200", choices=["vcfx_b200", "reference"])
     ap.add_argument("--variants", type=int, default=C2_VARIANTS, help="variants per GPU (default: full C2)")
@@ -641,7 +666,10 @@ def main():
     ap.add_argument("--no-cli", action="store_true")
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--configs", default="", help="comma-separated subset of C2,C3,C4 for the configs array")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the timed job computed in its last step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 0)
 
     if args.impl == "reference":
@@ -732,6 +760,9 @@ def main():
     clocks = sampler.stop()
     ms_total = e0.elapsed_time(e1)
     st_af, st_vc = ctx_af.sync(), ctx_vc.sync()
+    if args.dump_outputs:
+        dump_outputs(np, Path(args.dump_outputs), "" if world == 1 else f".rank{rank}",
+                     d_out[:int(st_af.bytes_out)].cpu().numpy().tobytes(), int(st_af.rows), int(st_vc.rows))
     t = torch.tensor([ms_total], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -823,7 +854,7 @@ def main():
         torch.cuda.synchronize()
         if world > 1:
             dist.barrier()
-        e2e_steps = max(3, min(args.steps, 5))
+        e2e_steps = args.steps
         torch.cuda.synchronize()
         t0 = time.perf_counter()
         for _ in range(e2e_steps):
@@ -891,6 +922,9 @@ def main():
         cpu = None
         if not args.no_cpu_baseline and world == 1:      # reported at N=1 only
             r = cpu_run or cpu_reference_run(CPU_SAMPLE_VARIANTS, 2, 1)
+            if not r:
+                log("[bench] reference tools not built (oracle/_ref/VCFX_*, make -C oracle ref REFERENCE=<VCFX source tree>): "
+                    "no cpu_baseline, and the parity entries compare with the oracle instead")
             if r:
                 cpu = {"value": r["gbps"], "unit": "GB/s", "cores": 1, "kind": "reference",
                        "sample": f"{r['variants']} variants x {SAMPLES} samples ({r['bytes'] / 1e9:.2f} GB) of the C2 stream, "

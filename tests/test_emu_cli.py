@@ -1,7 +1,8 @@
 """The host side of the five tools without a GPU: the real executables' sources (vcfx_b200/tools) linked against the
-emulator build of the library (tests/emu/), run through the cases of tests/test_gpu_cli.py against the compiled
-reference tools — with one context and with several contexts in one process (VCFX_CUDA_DEVICES: chunks dealt
-round-robin over the devices, text written in submission order)."""
+emulator build of the library (tests/emu/), run through the cases of tests/test_gpu_cli.py against the reference
+tools (tests/reference_runs.py: the reference build where there is one, else recorded outputs) — with one context and
+with several contexts in one process (VCFX_CUDA_DEVICES: chunks dealt round-robin over the devices, text written in
+submission order)."""
 import inspect
 import sys
 from pathlib import Path

@@ -1,5 +1,5 @@
-"""The five drop-in executables (vcfx_b200/bin/VCFX_*) against the compiled reference tools
-(oracle/_ref/VCFX_*): same argv, same stdin/file, stdout and exit code must be identical."""
+"""The drop-in executables (vcfx_b200/bin/VCFX_*) against the reference tools (tests/reference_runs.py: the reference
+build where there is one, else recorded outputs): same argv, same stdin/file, stdout and exit code must be identical."""
 import gzip
 import os
 import subprocess
@@ -7,13 +7,13 @@ from pathlib import Path
 
 import pytest
 
+import reference_runs
 import vcfgen
 from vcfx_b200 import synth
 
 pytestmark = pytest.mark.gpu
 ROOT = Path(__file__).resolve().parent.parent
 BIN = ROOT / "vcfx_b200" / "bin"
-REF = ROOT / "oracle" / "_ref"
 
 
 def run(exe, args, stdin=None, env=None):
@@ -25,15 +25,12 @@ def run(exe, args, stdin=None, env=None):
 
 
 def both(tool, args, stdin=None, env=None):
-    ref = REF / f"VCFX_{tool}"
-    if not ref.exists():
-        pytest.skip("oracle/_ref reference tools not built")
     mine = BIN / f"VCFX_{tool}"
     assert mine.exists(), f"{mine} not built (python -c 'import __graft_entry__ as g; g.build()')"
     a = run(mine, args, stdin, env)
-    b = run(ref, args, stdin)
+    b = reference_runs.run(tool, args, stdin)
     assert a[0] == b[0], (tool, args, a[0], b[0], a[2][-300:], b[2][-300:])
-    assert a[1] == b[1], (tool, args, a[1][:300], b[1][:300])
+    assert a[1] == b[1], (tool, args, a[1][:300], repr(b[1])[:300])
     return a, b
 
 
@@ -259,8 +256,8 @@ def test_allele_counter(tmp_path):
     both("allele_counter", ["-q", "-i", str(b)], env={"VCFX_CHUNK_BYTES": str(16 << 10)})
     # -z: the gzip container may differ, the payload may not
     mine = run(BIN / "VCFX_allele_counter", ["-q", "-z", "-i", str(a)])
-    ref = run(REF / "VCFX_allele_counter", ["-q", "-z", "-i", str(a)])
-    assert mine[0] == ref[0] == 0 and gzip.decompress(mine[1]) == gzip.decompress(ref[1])
+    ref = reference_runs.run("allele_counter", ["-q", "-z", "-i", str(a)])          # (its stdout: the payload of the reference's stream)
+    assert mine[0] == ref[0] == 0 and gzip.decompress(mine[1]) == ref[1]
     # header-less inputs
     both("allele_counter", ["-q"], stdin=b"##only\n")
     both("allele_counter", ["-q"], stdin=b"1\t1\t.\tA\tG\t.\t.\t.\tGT\t0/1\n")
@@ -270,8 +267,6 @@ def test_large_file_parallel_io(tmp_path):
     """Files past the 8 MiB mark take the multi-threaded pread / pwrite paths of the host reader:
     output to a regular file must be byte-identical to the reference's, with one and with eight I/O
     threads (VCFX_IO_THREADS), and identical to the pipe path."""
-    if not (REF / "VCFX_missing_detector").exists():
-        pytest.skip("oracle/_ref reference tools not built")
     src = tmp_path / "big.vcf"
     src.write_bytes(synth.make_vcf(3, 9000, 600, seed=21))          # ~ 22 MB, dots on most lines
     assert src.stat().st_size > (20 << 20)
@@ -283,9 +278,8 @@ def test_large_file_parallel_io(tmp_path):
         return r.returncode
 
     for tool, args in (("missing_detector", ["-q", "-t", "1", "-i", str(src)]), ("allele_freq_calc", ["-q", "-i", str(src)])):
-        ref_out = tmp_path / f"{tool}.ref"
-        assert to_file(REF / f"VCFX_{tool}", args, ref_out) == 0
-        want = ref_out.read_bytes()
+        rc, want, _ = reference_runs.run(tool, args)
+        assert rc == 0
         for threads in ("1", "8"):
             out = tmp_path / f"{tool}.{threads}"
             assert to_file(BIN / f"VCFX_{tool}", args, out, {"VCFX_IO_THREADS": threads}) == 0

@@ -1,12 +1,14 @@
 """The oracle (CPU restatement, oracle/vcfx_oracle.c) against the committed outputs of the reference
-tools, and — when the reference binaries are present — against those binaries on fresh seeded inputs.
-This is what pins the oracle; the GPU parity tests then compare the CUDA path with the oracle."""
+tools (tests/golden/reference_outputs.json), and on seeded inputs against tests/reference_runs.py: the reference
+build where there is one, else outputs recorded from the drop-in tools (see there).  This is what pins the oracle;
+the GPU parity tests then compare the CUDA path with the oracle."""
 import os
 import tempfile
 
 import pytest
 
 import golden_util
+import reference_runs
 import vcfgen
 from vcfx_b200 import synth
 
@@ -81,85 +83,81 @@ def test_golden_covers_the_modes_that_differ():
 
 @pytest.mark.parametrize("seed", range(25))
 def test_oracle_matches_reference_binaries_fuzz(oracle, seed):
-    """Fresh inputs against oracle/_ref/VCFX_* (skipped where the reference could not be built)."""
+    """Seeded inputs against the reference tools (tests/reference_runs.py)."""
     O = oracle
-    if not O.have_reference():
-        pytest.skip("oracle/_ref reference tools not built")
     hdr = ["normal", "normal", "late", "none", "double"][seed % 5]
     data = vcfgen.make_vcf(9000 + seed, n_lines=30, n_samples=1 + seed % 7, crlf=(seed % 7 == 3), final_newline=(seed % 5 != 2), header=hdr)
     with tempfile.NamedTemporaryFile(suffix=".vcf") as f:
         f.write(data); f.flush()
         for tool, fn in (("allele_freq_calc", O.allele_freq), ("hwe_tester", O.hwe), ("missing_detector", O.missing)):
             extra = ["-t", "1"] if tool == "missing_detector" else []
-            rc, out, _ = O.run_ref(tool, ["-q", *extra, "-i", f.name]); r = fn(data, O.FILE)
+            rc, out, _ = reference_runs.run(tool, ["-q", *extra, "-i", f.name]); r = fn(data, O.FILE)
             assert (r.rc, r.out) == (rc, out), (tool, "file")
-            rc, out, _ = O.run_ref(tool, ["-q"] if tool != "hwe_tester" else [], stdin=data); r = fn(data, O.STDIN)
+            rc, out, _ = reference_runs.run(tool, ["-q"] if tool != "hwe_tester" else [], stdin=data); r = fn(data, O.STDIN)
             assert (r.rc, r.out) == (rc, out), (tool, "stdin")
-        rc, out, err = O.run_ref("indexer", [f.name]); r = O.indexer(data, O.FILE)
+        rc, out, err = reference_runs.run("indexer", [f.name]); r = O.indexer(data, O.FILE)
         assert (r.rc, r.out, r.warnings) == (rc, out, err.count(b"no #CHROM")), "indexer file"
-        rc, out, err = O.run_ref("indexer", [], stdin=data); r = O.indexer(data, O.STDIN)
+        rc, out, err = reference_runs.run("indexer", [], stdin=data); r = O.indexer(data, O.STDIN)
         assert (r.rc, r.out, r.warnings) == (rc, out, err.count(b"no #CHROM")), "indexer stdin"
-        rc, out, err = O.run_ref("nonref_filter", ["-i", f.name]); r = O.nonref_filter(data, O.FILE)
+        rc, out, err = reference_runs.run("nonref_filter", ["-i", f.name]); r = O.nonref_filter(data, O.FILE)
         assert (r.rc, r.out, r.warnings) == (rc, out, err.count(b"Warning")), "nonref_filter file"
-        rc, out, err = O.run_ref("nonref_filter", [], stdin=data); r = O.nonref_filter(data, O.STDIN)
+        rc, out, err = reference_runs.run("nonref_filter", [], stdin=data); r = O.nonref_filter(data, O.STDIN)
         assert (r.rc, r.out, r.warnings) == (rc, out, err.count(b"Warning")), "nonref_filter stdin"
-        rc, out, err = O.run_ref("phase_checker", ["-i", f.name]); r = O.phase_checker(data, O.FILE)
+        rc, out, err = reference_runs.run("phase_checker", ["-i", f.name]); r = O.phase_checker(data, O.FILE)
         assert (r.rc, r.out, O.phase_checker_stderr(data, O.FILE)) == (rc, out, err), "phase_checker file"
-        rc, out, err = O.run_ref("phase_checker", ["-"], stdin=data); r = O.phase_checker(data, O.STDIN)
+        rc, out, err = reference_runs.run("phase_checker", ["-"], stdin=data); r = O.phase_checker(data, O.STDIN)
         assert (r.rc, r.out, O.phase_checker_stderr(data, O.STDIN)) == (rc, out, err), "phase_checker stdin"
-        rc, out, err = O.run_ref("phase_checker", ["-q"], stdin=data)
+        rc, out, err = reference_runs.run("phase_checker", ["-q"], stdin=data)
         assert (rc, out, err) == (r.rc, r.out, b""), "phase_checker -q"
-        rc, out, err = O.run_ref("dosage_calculator", ["-i", f.name]); r = O.dosage(data, O.FILE)
+        rc, out, err = reference_runs.run("dosage_calculator", ["-i", f.name]); r = O.dosage(data, O.FILE)
         assert (r.rc, r.out, O.DS_ERROR if r.first_bad_line else O.DS_WARNING * r.warnings) == (rc, out, err), "dosage_calculator file"
-        rc, out, err = O.run_ref("dosage_calculator", ["-q"], stdin=data); r = O.dosage(data, O.STDIN)
+        rc, out, err = reference_runs.run("dosage_calculator", ["-q"], stdin=data); r = O.dosage(data, O.STDIN)
         assert (r.rc, r.out, O.DS_ERROR if r.first_bad_line else O.DS_WARNING * r.warnings) == (rc, out, err), "dosage_calculator stdin"
         for q, strict in (("0/1", False), ("1|1", True), ("2/0", False)):
             a = ["-g", q] + (["--strict"] if strict else [])
-            rc, out, err = O.run_ref("genotype_query", [*a, "-i", f.name]); r, e = O.genotype_query(data, q, O.FILE, strict)
+            rc, out, err = reference_runs.run("genotype_query", [*a, "-i", f.name]); r, e = O.genotype_query(data, q, O.FILE, strict)
             assert (r.rc, r.out, e) == (rc, out, err), ("genotype_query file", a)
-            rc, out, err = O.run_ref("genotype_query", a, stdin=data); r, e = O.genotype_query(data, q, O.STDIN, strict)
+            rc, out, err = reference_runs.run("genotype_query", a, stdin=data); r, e = O.genotype_query(data, q, O.STDIN, strict)
             assert (r.rc, r.out, e) == (rc, out, err), ("genotype_query stdin", a)
         for flags, args in ((0, []), (O.IB_GLOBAL, ["--freq-mode", "global"]), (O.IB_SKIP_BOUNDARY, ["--skip-boundary"]),
                             (O.IB_SKIP_BOUNDARY | O.IB_COUNT_BOUNDARY, ["--skip-boundary", "--count-boundary-as-used"])):
-            rc, out, err = O.run_ref("inbreeding_calculator", ["-q", *args, "-i", f.name]); r = O.inbreeding(data, O.FILE, flags | O.IB_QUIET)
+            rc, out, err = reference_runs.run("inbreeding_calculator", ["-q", *args, "-i", f.name]); r = O.inbreeding(data, O.FILE, flags | O.IB_QUIET)
             assert (r.rc, r.out, O.IB_MESSAGES[r.warnings]) == (rc, out, err), ("inbreeding_calculator file", args)
-            rc, out, err = O.run_ref("inbreeding_calculator", ["-q", *args], stdin=data); r = O.inbreeding(data, O.STDIN, flags | O.IB_QUIET)
+            rc, out, err = reference_runs.run("inbreeding_calculator", ["-q", *args], stdin=data); r = O.inbreeding(data, O.STDIN, flags | O.IB_QUIET)
             assert (r.rc, r.out, O.IB_MESSAGES[r.warnings]) == (rc, out, err), ("inbreeding_calculator stdin", args)
         for strict in (False, True):
             a = ["--strict"] if strict else []
-            rc, out, err = O.run_ref("variant_counter", [*a, f.name]); r = O.variant_count(data, O.FILE, strict)
+            rc, out, err = reference_runs.run("variant_counter", [*a, f.name]); r = O.variant_count(data, O.FILE, strict)
             assert (r.rc, r.out) == (rc, out)
             if strict and rc:
                 assert b"line %d " % r.first_bad_line in err
         data = vcfgen.make_vcf(9100 + seed, n_lines=30, n_samples=1 + seed % 7, domain="ac", final_newline=(seed % 5 != 2), header=hdr)
         f.seek(0); f.truncate(); f.write(data); f.flush()
-        rc, out, _ = O.run_ref("allele_counter", ["-q", "-i", f.name]); r = O.allele_counter(data, O.AC_MT_TEXT)
+        rc, out, _ = reference_runs.run("allele_counter", ["-q", "-i", f.name]); r = O.allele_counter(data, O.AC_MT_TEXT)
         assert (r.rc, r.out) == (rc, out)
-        rc, out, _ = O.run_ref("allele_counter", ["-q"], stdin=data); r = O.allele_counter(data, O.AC_STREAM)
+        rc, out, _ = reference_runs.run("allele_counter", ["-q"], stdin=data); r = O.allele_counter(data, O.AC_STREAM)
         assert (r.rc, r.out) == (rc, out)
-        rc, out, _ = O.run_ref("allele_counter", ["-q", "-a", "-i", f.name]); r = O.allele_counter(data, O.AC_UNIFIED, O.AC_AGGREGATE)
+        rc, out, _ = reference_runs.run("allele_counter", ["-q", "-a", "-i", f.name]); r = O.allele_counter(data, O.AC_UNIFIED, O.AC_AGGREGATE)
         assert (r.rc, r.out) == (rc, out)
 
 
 def test_oracle_matches_reference_binaries_shapes(oracle):
     O = oracle
-    if not O.have_reference():
-        pytest.skip("oracle/_ref reference tools not built")
     for shape, V, S in ((1, 400, 100), (2, 60, 2504), (3, 60, 2504), (4, 150, 33)):
         data = synth.make_vcf(shape, V, S, seed=shape)
         with tempfile.NamedTemporaryFile(suffix=".vcf") as f:
             f.write(data); f.flush()
             for tool, fn in (("allele_freq_calc", O.allele_freq), ("hwe_tester", O.hwe), ("missing_detector", O.missing)):
                 extra = ["-t", "1"] if tool == "missing_detector" else []
-                rc, out, _ = O.run_ref(tool, ["-q", *extra, "-i", f.name], timeout=60)
+                rc, out, _ = reference_runs.run(tool, ["-q", *extra, "-i", f.name])
                 assert (fn(data, O.FILE).out) == out, (shape, tool)
-            rc, out, _ = O.run_ref("variant_counter", [f.name])
+            rc, out, _ = reference_runs.run("variant_counter", [f.name])
             assert O.variant_count(data).out == out
-            rc, out, _ = O.run_ref("nonref_filter", ["-i", f.name], timeout=60)
+            rc, out, _ = reference_runs.run("nonref_filter", ["-i", f.name])
             assert O.nonref_filter(data, O.FILE).out == out, (shape, "nonref_filter")
-            rc, out, err = O.run_ref("inbreeding_calculator", ["-q", "-i", f.name], timeout=60)
+            rc, out, err = reference_runs.run("inbreeding_calculator", ["-q", "-i", f.name])
             assert O.inbreeding(data, O.FILE, O.IB_QUIET).out == out, (shape, "inbreeding_calculator")
-            rc, out, err = O.run_ref("phase_checker", ["-i", f.name], timeout=60)
+            rc, out, err = reference_runs.run("phase_checker", ["-i", f.name])
             assert (O.phase_checker(data, O.FILE).out, O.phase_checker_stderr(data, O.FILE)) == (out, err), (shape, "phase_checker")
 
 
