@@ -79,18 +79,41 @@ def run_all(api, O, data, tag, chunk_bytes=0, tile_bytes=0, tools=("af", "hwe", 
                     assert len(r.totals.short_line_numbers) == o.warnings
 
 
-@pytest.mark.parametrize("shape,V,S", [(1, 2000, 100), (2, 200, 2504), (3, 200, 2504), (4, 40, 2504),
-                                       (2, 3000, 7), (3, 3000, 33), (4, 500, 21), (1, 1, 1), (2, 50, 0)])
+# the inputs below are shared with test_gpu_resident.py, which runs them through the device-resident entry point
+SHAPES = [(1, 2000, 100), (2, 200, 2504), (3, 200, 2504), (4, 40, 2504), (2, 3000, 7), (3, 3000, 33), (4, 500, 21), (1, 1, 1), (2, 50, 0)]
+
+
+def shape_input(shape, V, S):
+    return synth.make_vcf(shape, V, S, seed=100 + shape)
+
+
+def adversarial_input(seed):
+    """vcfgen: both header kinds and the broken ones, CRLF, no final newline."""
+    hdr = ["normal", "normal", "late", "none", "double"][seed % 5]
+    return vcfgen.make_vcf(seed, n_lines=60, n_samples=1 + seed % 9, crlf=(seed % 7 == 3),
+                           final_newline=(seed % 4 != 1), header=hdr)
+
+
+DEGENERATE = (b"", b"\n", b"\n\n\n", b"#only header\n", b"#CHROM\tPOS\n", b"1\t2\t3", b"\t\t\t\t\t\t\t\tGT\n",
+              b"#CHROM\n\t\t\t\t\t\t\t\tGT", b"#CHROM\n1\t1\t.\tA\tG\t.\t.\t.\tGT\t0/1\r\n",
+              b"#CHROM\n1\t1\t.\tA\tG\t.\t.\t.\tGT\t\n", b"#CHROM\n1\t1\t.\tA\tG\t.\t.\t.\tGT\t0/1\t")
+
+SWEEP_S = list(range(1, 34, 2)) + list(range(100, 134, 3)) + [119, 120, 121, 127, 128, 129, 255, 256, 257, 383, 511, 640]
+
+
+def sweep_input(shape, S):
+    return synth.make_vcf(shape, 150 if S < 300 else 40, S, seed=1000 * shape + S)
+
+
+@pytest.mark.parametrize("shape,V,S", SHAPES)
 def test_synthetic_shapes(cuda_api, oracle, shape, V, S):
-    data = synth.make_vcf(shape, V, S, seed=100 + shape)
+    data = shape_input(shape, V, S)
     run_all(cuda_api, oracle, data, f"shape{shape} {V}x{S}")
 
 
 @pytest.mark.parametrize("seed", range(40))
 def test_adversarial(cuda_api, oracle, seed):
-    hdr = ["normal", "normal", "late", "none", "double"][seed % 5]
-    data = vcfgen.make_vcf(seed, n_lines=60, n_samples=1 + seed % 9, crlf=(seed % 7 == 3),
-                           final_newline=(seed % 4 != 1), header=hdr)
+    data = adversarial_input(seed)
     run_all(cuda_api, oracle, data, f"fuzz{seed}")
 
 
@@ -114,9 +137,7 @@ def test_multi_chunk_stream(cuda_api, oracle):
 
 
 def test_empty_and_degenerate(cuda_api, oracle):
-    for data in (b"", b"\n", b"\n\n\n", b"#only header\n", b"#CHROM\tPOS\n", b"1\t2\t3", b"\t\t\t\t\t\t\t\tGT\n",
-                 b"#CHROM\n\t\t\t\t\t\t\t\tGT", b"#CHROM\n1\t1\t.\tA\tG\t.\t.\t.\tGT\t0/1\r\n",
-                 b"#CHROM\n1\t1\t.\tA\tG\t.\t.\t.\tGT\t\n", b"#CHROM\n1\t1\t.\tA\tG\t.\t.\t.\tGT\t0/1\t"):
+    for data in DEGENERATE:
         run_all(cuda_api, oracle, data, repr(data[:20]))
 
 
@@ -245,8 +266,8 @@ def test_line_lengths_sweep(cuda_api, oracle):
     the first bytes of the next one, phase shifts (haploid / missing calls) right before a window or
     line end — the places where the lattice tiers hand over to the exact path."""
     for shape in (1, 2, 3):
-        for S in list(range(1, 34, 2)) + list(range(100, 134, 3)) + [119, 120, 121, 127, 128, 129, 255, 256, 257, 383, 511, 640]:
-            data = synth.make_vcf(shape, 150 if S < 300 else 40, S, seed=1000 * shape + S)
+        for S in SWEEP_S:
+            data = sweep_input(shape, S)
             run_all(cuda_api, oracle, data, f"sweep shape{shape} S{S}", tools=("af", "hwe"))
     data = synth.make_vcf(3, 3000, 120, seed=13)
     run_all(cuda_api, oracle, data, "sweep regression S120", chunk_bytes=256 << 10)
@@ -419,12 +440,17 @@ def test_phase_checker_cases(cuda_api, oracle):
         run_all(cuda_api, oracle, data, f"pc S{S} tile512", tile_bytes=512, tools=("pc",))
 
 
+def pc_dropped_lines_input():
+    """(input, lines phase_checker drops): 2^20 + 5000 short lines, more than the first event list holds."""
+    hdr = b"##fileformat=VCFv4.2\n#CHROM\tPOS\tID\tREF\tALT\tQUAL\tFILTER\tINFO\tFORMAT\tA\n"
+    n = (1 << 20) + 5000
+    return hdr + b"1\t2\n" * n + b"1\t7\t.\tA\tG\t.\t.\t.\tGT\t0|1\n", n
+
+
 def test_phase_checker_more_dropped_lines_than_the_event_list(cuda_api, oracle):
     """Every dropped line is reported; the list starts with room for 2^20 of them and the chunk is run again with a longer
     one when that is not enough."""
-    hdr = b"##fileformat=VCFv4.2\n#CHROM\tPOS\tID\tREF\tALT\tQUAL\tFILTER\tINFO\tFORMAT\tA\n"
-    n = (1 << 20) + 5000
-    data = hdr + b"1\t2\n" * n + b"1\t7\t.\tA\tG\t.\t.\t.\tGT\t0|1\n"
+    data, n = pc_dropped_lines_input()
     r = cuda_api.phase_checker(data, 0)
     o = oracle.phase_checker(data, 0)
     assert r.out == o.out and r.totals.flagged == n
@@ -518,12 +544,7 @@ def test_inbreeding_calculator_cases(cuda_api, oracle):
         run_all(cuda_api, oracle, data, f"ib lattice S{S} tile512", tile_bytes=512, tools=("ib",))
     # thousands of samples in the header, two columns on most lines: more rows x samples than the panels were sized for — the
     # chunk is run again with larger ones, and the chunks behind it (already launched) wait their turn and are run again too
-    S = 4000
-    hdr = b"##f\n#CHROM\tP\tI\tR\tA\tQ\tF\tI\tFORMAT\t" + b"\t".join(b"N%d" % i for i in range(S)) + b"\n"
-    g = [b"0/1", b"1/1", b"0/0", b"0|1", b"./."]
-    lines = [b"1\t%d\t.\tA\tG\t.\t.\t.\tGT\t%s\t%s" % (k + 1, g[k % 5], g[(k * 3 + 1) % 5]) for k in range(2500)]
-    lines[7] += b"\t" + b"\t".join(g[(j * 7) % 5] for j in range(S - 2))
-    data = hdr + b"\n".join(lines) + b"\n"
+    data = ib_few_columns_input()
     for kw in ({"chunk_bytes": 16 << 10}, {}):
         run_all(cuda_api, oracle, data, f"ib few columns {kw}", tools=("ib",), **kw)
     # a context is good for one stream after the other: the sums start again behind a final chunk
@@ -542,16 +563,29 @@ def test_inbreeding_calculator_cases(cuda_api, oracle):
     ctx.close()
 
 
-def test_allele_counter_two_digit_counts(cuda_api, oracle):
-    """allele_counter TEXT rows are sized without looking at the genotypes (one digit per count); a
-    sample with ten or more alleles of a kind, or 128+ (int8 wrap to a negative number), breaks that
-    guess: the write pass notices and the chunk is run again with exact sizes."""
+def ib_few_columns_input():
+    S = 4000
+    hdr = b"##f\n#CHROM\tP\tI\tR\tA\tQ\tF\tI\tFORMAT\t" + b"\t".join(b"N%d" % i for i in range(S)) + b"\n"
+    g = [b"0/1", b"1/1", b"0/0", b"0|1", b"./."]
+    lines = [b"1\t%d\t.\tA\tG\t.\t.\t.\tGT\t%s\t%s" % (k + 1, g[k % 5], g[(k * 3 + 1) % 5]) for k in range(2500)]
+    lines[7] += b"\t" + b"\t".join(g[(j * 7) % 5] for j in range(S - 2))
+    return hdr + b"\n".join(lines) + b"\n"
+
+
+def two_digit_counts_input():
     hdr = b"##fileformat=VCFv4.2\n#CHROM\tPOS\tID\tREF\tALT\tQUAL\tFILTER\tINFO\tFORMAT\tA\tB\tC\n"
     deca = b"/".join([b"0"] * 10)
     wrap = b"|".join([b"1"] * 130)
     body = b"".join(b"1\t%d\trs%d\tA\tG\t.\tPASS\t.\tGT\t0|1\t%s\t1/1\n" % (100 + i, i, deca if i % 7 == 3 else (wrap if i % 11 == 5 else b"0/0"))
                     for i in range(60))
-    data = hdr + body
+    return hdr + body
+
+
+def test_allele_counter_two_digit_counts(cuda_api, oracle):
+    """allele_counter TEXT rows are sized without looking at the genotypes (one digit per count); a
+    sample with ten or more alleles of a kind, or 128+ (int8 wrap to a negative number), breaks that
+    guess: the write pass notices and the chunk is run again with exact sizes."""
+    data = two_digit_counts_input()
     for kw in ({}, {"chunk_bytes": 4096}, {"tile_bytes": 512}):
         o = oracle.allele_counter(data)
         r = cuda_api.allele_counter(data, **kw)
@@ -562,14 +596,19 @@ def test_allele_counter_two_digit_counts(cuda_api, oracle):
     _cmp("ac after exact", cuda_api.allele_counter(data2).out, oracle.allele_counter(data2).out)
 
 
+def more_rows_input():
+    """130,000 lines of 36 bytes: more rows than the default record capacity of a 4 MiB chunk."""
+    hdr = b"##fileformat=VCFv4.2\n#CHROM\tPOS\tID\tREF\tALT\tQUAL\tFILTER\tINFO\tFORMAT\tA\tB\n"
+    gts = [b"0|1", b"1|1", b"0|0", b"./.", b"1|0"]
+    body = b"".join(b"1\t%d\t.\tA\tG\t.\t.\t.\tGT\t%s\t%s\n" % (i + 1, gts[i % 5], gts[(i * 7 + 3) % 5]) for i in range(130000))
+    return hdr + body
+
+
 def test_more_rows_than_the_default_record_capacity(cuda_api, oracle):
     """Row records are sized for one row per 256 input bytes (+64 Ki); a chunk of very short lines has
     more: the launch reports it and is repeated with the exact count (block-wise slot reservation
     included), through the streaming path and through several chunks."""
-    hdr = b"##fileformat=VCFv4.2\n#CHROM\tPOS\tID\tREF\tALT\tQUAL\tFILTER\tINFO\tFORMAT\tA\tB\n"
-    gts = [b"0|1", b"1|1", b"0|0", b"./.", b"1|0"]
-    body = b"".join(b"1\t%d\t.\tA\tG\t.\t.\t.\tGT\t%s\t%s\n" % (i + 1, gts[i % 5], gts[(i * 7 + 3) % 5]) for i in range(130000))
-    data = hdr + body
+    data = more_rows_input()
     chunk = 4 << 20                                       # the slot's capacity is sized from the chunk size
     assert len(data) <= chunk and chunk // 256 + 65536 < 130000
     run_all(cuda_api, oracle, data, "many short lines, one 4 MiB chunk", chunk_bytes=chunk, tools=("af", "hwe", "md", "vc"))
