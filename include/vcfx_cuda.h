@@ -65,7 +65,14 @@ typedef enum {
     VCFX_OP_DOSAGE         = 10,  /* VCFX_dosage_calculator.cpp:375-591 processFileMmap, :209-366 calculateDosage (SURVEY §8 f2): a row
                                      "CHROM..ALT \t d,d,NA,.." per data line with ten columns; stats.short_lines = lines with fewer
                                      (one warning each).  The caller prints the header row and ends the run at a data line that
-                                     comes before the "#CHROM" line */
+                                     comes before the "#CHROM" line.
+                                     VCFX_F_DS_MATRIX: the same rows as a matrix instead of text, cfg.n_sel = W sample columns
+                                     (0 is valid).  Output of a launch / chunk: rows x vcfx_ds_row, then at byte 16 x rows the
+                                     rows x W int8 codes, row-major: 0 / 1 / 2 the dosage the text prints, -1 its "NA" (every
+                                     column of a line without a GT key too), -2 for a column s >= n_cols the line does not have.
+                                     Columns beyond W are dropped (n_cols keeps the true count; stats.flagged counts such rows).
+                                     stats.rows = rows, stats.bytes_out = rows x (16 + W); short_lines, data_lines as for the text.
+                                     run_device wants d_out 16-byte aligned (else VCFX_E_INVALID) */
     VCFX_OP_INDEX          = 6,   /* VCFX_indexer.cpp:205-322 createVCFIndexMmap, :329-443 createVCFIndex (SURVEY §8 f4) */
     VCFX_OP_NONREF_FILTER  = 5    /* VCFX_nonref_filter.cpp:458-548 filterNonRefMmap, :553-631 filterNonRef (SURVEY §8 f2) */
 } vcfx_op;
@@ -87,13 +94,14 @@ typedef enum {
     VCFX_E_UNSUPPORTED    = -8
 } vcfx_err;
 
-/* allele_counter variants (cfg.flags) */
+/* variants of an op (cfg.flags): the bits are per op */
 #define VCFX_F_GQ_STRICT         0x01u  /* genotype_query --strict: byte-for-byte comparison (:277-279)               */
 #define VCFX_F_IB_GLOBAL         0x01u  /* inbreeding_calculator --freq-mode global (:596-604)                 */
 #define VCFX_F_IB_SKIP_BOUNDARY  0x02u  /* --skip-boundary (:614-620)                                          */
 #define VCFX_F_IB_COUNT_BOUNDARY 0x04u  /* --count-boundary-as-used                                            */
 #define VCFX_F_AC_AGGREGATE   0x01u  /* -a: one row per variant (countAllelesUnified :1440-1461)          */
 #define VCFX_F_AC_BINARY      0x02u  /* -b: int8 {ref,alt} per selected sample (:1444-1449)               */
+#define VCFX_F_DS_MATRIX      0x01u  /* dosage_calculator: int8 variants x samples matrix instead of text (see VCFX_OP_DOSAGE) */
 #define VCFX_F_AC_FORWARD     0x04u  /* stdin / unified column walk: forward only, stop at the first absent
                                         column (:1222-1229, :1416-1423); without it: processChunk's random
                                         access with 0/0 padding and int8 storage (:610-627)               */
@@ -115,6 +123,13 @@ typedef struct {
     const char     *sel_names;      /* concatenated names, each followed by '\t'                */
     const uint32_t *sel_name_off;   /* [n_sel + 1] offsets into sel_names                       */
 } vcfx_cfg;
+
+/* VCFX_OP_DOSAGE with VCFX_F_DS_MATRIX: the metadata of one matrix row (16 bytes, the rows in file order) */
+typedef struct vcfx_ds_row {
+    uint64_t line_offset;      /* offset of the row's line in the whole input: info.file_offset + offset in the chunk */
+    uint32_t n_cols;           /* sample columns of the line (may exceed W)                                           */
+    uint32_t flags;            /* bit 0: the line has no GT key (the text prints "NA" alone; every code is -1)         */
+} vcfx_ds_row;
 
 /* what the caller knows about the chunk it submits */
 typedef struct {

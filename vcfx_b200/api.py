@@ -152,7 +152,7 @@ class Context:
 
     def __init__(self, op: int, mode: int = FILE, device: int = 0, flags: int = 0, chunk_bytes: int = 0,
                  out_bytes: int = 0, n_slots: int = 0, tile_bytes: int = 0, stream: int | None = None,
-                 sel_cols=None, sel_names=None, query: bytes | None = None):
+                 sel_cols=None, sel_names=None, query: bytes | None = None, width: int | None = None):
         self._l = load()
         self._h = C.c_void_p()
         cfg = Cfg(device=device, op=op, mode=mode, flags=flags, chunk_bytes=chunk_bytes, out_bytes=out_bytes,
@@ -171,6 +171,8 @@ class Context:
         if query is not None:                      # genotype_query: the -g argument travels in sel_names, its length in n_sel
             cfg.n_sel = len(query); cfg.sel_names = query
             self._keep = [query]
+        if width is not None:                      # dosage_calculator matrix mode: W, the sample columns of the matrix
+            cfg.n_sel = int(width)
         self._check(self._l.vcfx_cuda_create(C.byref(cfg), C.byref(self._h)))
         self.op, self.mode = op, mode
 
@@ -565,13 +567,11 @@ DS_WARNING = b"Warning: Skipping VCF line with fewer than 10 fields.\n"
 DS_ERROR = b"Error: VCF header (#CHROM) not found before variant records.\n"
 
 
-def dosage_calculator(data: bytes, mode: int = FILE, quiet: bool = False, chunk_bytes: int = 0, **kw) -> ToolResult:
-    """VCFX_dosage_calculator: per data line "CHROM..ALT \\t d,d,NA,.." (processFileMmap :375-591, calculateDosage :209-366).
-    A data line in front of the "#CHROM" line ends the run with nothing on stdout (exit code 1 in file mode); an empty FILE
-    gives nothing at all; stdin mode prints its warnings even with -q."""
-    if mode == FILE and len(data) == 0:
-        return ToolResult(b"", 0, Totals())
-    pos, n, found = 0, len(data), False
+def _ds_prescan(data, mode: int):
+    """dosage_calculator's host rule, applied to the lines up to the first data line: (offset of the first data line or
+    len(data), whether a "#CHROM" line came before it, the sample names of the first "#CHROM" line — its columns from index
+    9, a '\\r' in front of the '\\n' and an empty column behind a final tab left out)."""
+    pos, n, found, names = 0, len(data), False, []
     while pos < n:                                       # up to the first data line
         nl = data.find(b"\n", pos)
         le = n if nl < 0 else nl
@@ -580,15 +580,135 @@ def dosage_calculator(data: bytes, mode: int = FILE, quiet: bool = False, chunk_
             line = line[:-1]
         if line:
             if not line.startswith(b"#"):
-                if not found:
-                    return ToolResult(b"", 1 if mode == FILE else 0, Totals(), DS_ERROR)
-                break
-            if line.startswith(b"#CHROM"):
+                return pos, found, names
+            if line.startswith(b"#CHROM") and not found:
                 found = True
+                f = bytes(line[:-1] if (mode != FILE and line.endswith(b"\r")) else line).split(b"\t")[9:]
+                names = f[:-1] if f and f[-1] == b"" else f
         pos = le + 1
+    return n, found, names
+
+
+def dosage_calculator(data: bytes, mode: int = FILE, quiet: bool = False, chunk_bytes: int = 0, **kw) -> ToolResult:
+    """VCFX_dosage_calculator: per data line "CHROM..ALT \\t d,d,NA,.." (processFileMmap :375-591, calculateDosage :209-366).
+    A data line in front of the "#CHROM" line ends the run with nothing on stdout (exit code 1 in file mode); an empty FILE
+    gives nothing at all; stdin mode prints its warnings even with -q."""
+    if mode == FILE and len(data) == 0:
+        return ToolResult(b"", 0, Totals())
+    first_data, found, _ = _ds_prescan(data, mode)
+    if first_data < len(data) and not found:
+        return ToolResult(b"", 1 if mode == FILE else 0, Totals(), DS_ERROR)
     body, tot = _run(OP_DOSAGE, data, mode, chunk_bytes, **kw)
     warn = b"" if (quiet and mode == FILE) else DS_WARNING * tot.short_lines
     return ToolResult(DS_HEADER + body, 0, tot, warn)
+
+
+F_DS_MATRIX = 1
+DS_ROW_BYTES = 16                                      # vcfx_ds_row: uint64 line_offset, uint32 n_cols, uint32 flags
+
+
+@dataclass
+class DosageMatrix:
+    """dosage_calculator's rows as numbers: row i is the row the tool prints for the line at byte line_offset[i].
+    codes[i, s] = 0 / 1 / 2 the dosage, -1 "NA" (every column of a line without a GT key too), -2 the line has no column s;
+    columns beyond the width are dropped (n_cols keeps the true count, totals.flagged counts such rows)."""
+    samples: list                  # the "#CHROM" line's columns from index 9
+    codes: object                  # int8 [rows, W]
+    line_offset: object            # int64 [rows]
+    n_cols: object                 # int32 [rows]
+    no_gt: object                  # bool [rows]: the line has no GT key (the tool prints "NA" alone)
+    totals: Totals
+    err: bytes = b""               # the warnings the tool prints on stderr
+
+
+def _ds_matrix_prescan(data, mode: int):
+    """(sample names) after dosage_calculator's host rule: a data line in front of the "#CHROM" line ends the tool's run."""
+    first_data, found, names = _ds_prescan(data, mode)
+    if first_data < len(data) and not found:
+        raise VcfxCudaError(-1, DS_ERROR.decode().rstrip("\n"))
+    return names
+
+
+def _ds_split(piece: bytes, width: int):
+    """(metadata, codes) numpy views of one chunk's matrix output."""
+    import numpy as np
+    rows = len(piece) // (DS_ROW_BYTES + width)
+    meta = np.frombuffer(piece, dtype=np.dtype([("line_offset", "<u8"), ("n_cols", "<u4"), ("flags", "<u4")]), count=rows)
+    codes = np.frombuffer(piece, dtype=np.int8, count=rows * width, offset=DS_ROW_BYTES * rows).reshape(rows, width)
+    return meta, codes
+
+
+def dosage_matrix(data: bytes, mode: int = FILE, width: int | None = None, chunk_bytes: int = 0, **kw) -> DosageMatrix:
+    """dosage_calculator's genotypes as an int8 variants x samples matrix (CPU tensors), through the streaming path.  The
+    width defaults to the number of samples of the "#CHROM" line.  Raises VcfxCudaError with the tool's error text when a
+    data line comes before the "#CHROM" line."""
+    import numpy as np
+    import torch
+    names = [] if (mode == FILE and len(data) == 0) else _ds_matrix_prescan(data, mode)
+    W = len(names) if width is None else int(width)
+    metas, codes, tot = [], [], Totals()
+    if len(data):
+        chunk_bytes = chunk_bytes or min(64 << 20, max(1 << 20, (len(data) + (1 << 20) - 1) & ~((1 << 20) - 1)))
+        ctx, cached = _cached_context(OP_DOSAGE, mode, 0, F_DS_MATRIX, chunk_bytes, width=W, **kw)
+        try:
+            outs, tot = stream_bytes(ctx, data, chunk_bytes)
+        except Exception:
+            if cached:
+                _ctx_cache.pop(next(k for k, v in _ctx_cache.items() if v is ctx), None)
+            ctx.close()
+            raise
+        for piece in outs:
+            m, c = _ds_split(piece, W)
+            metas.append(m); codes.append(c)
+    meta = np.concatenate(metas) if metas else _ds_split(b"", W)[0]
+    code = np.concatenate(codes) if codes else np.zeros((0, W), dtype=np.int8)
+    return DosageMatrix(names, torch.from_numpy(np.ascontiguousarray(code)), torch.from_numpy(meta["line_offset"].astype(np.int64)),
+                        torch.from_numpy(meta["n_cols"].astype(np.int32)), torch.from_numpy((meta["flags"] & 1).astype(bool)),
+                        tot, DS_WARNING * tot.short_lines)
+
+
+def _ds_device_head(d_in, nbytes: int, mode: int):
+    """The sample names, read back from the leading lines of a device input only: the bytes up to the first data line."""
+    k = min(nbytes, 1 << 16)
+    while True:
+        head = d_in[:k].cpu().numpy().tobytes()
+        cut = k if k == nbytes else head.rfind(b"\n") + 1         # complete lines only, unless that is the whole input
+        first_data, _, _ = _ds_prescan(head[:cut], mode)
+        if first_data < cut or k == nbytes:
+            return _ds_matrix_prescan(head[:cut], mode)
+        k = min(nbytes, 4 * k)
+
+
+def dosage_matrix_device(d_in, nbytes: int, mode: int = FILE, width: int | None = None, line_hint: int = 0) -> DosageMatrix:
+    """dosage_matrix for an input already on the device: d_in is a uint8 CUDA tensor of at least nbytes + DEVICE_PAD bytes
+    (16-byte aligned).  Only the leading '#' block comes back to the host.  The output is sized from a newline count on
+    the device (rows <= lines) and the library runs on torch.cuda.current_stream(), so torch work behind it is ordered
+    after it; codes, line_offset, n_cols and no_gt are views into one output tensor on the same device."""
+    import torch
+    if d_in.dtype != torch.uint8 or not d_in.is_cuda or d_in.numel() < nbytes + DEVICE_PAD or d_in.data_ptr() % 16:
+        raise VcfxCudaError(-1, "d_in must be a 16-byte aligned uint8 CUDA tensor of at least nbytes + DEVICE_PAD bytes")
+    names = [] if (mode == FILE and nbytes == 0) else _ds_device_head(d_in, nbytes, mode)
+    W = len(names) if width is None else int(width)
+    lines = 1
+    for s in range(0, nbytes, 1 << 28):                     # (bounded temporaries for inputs of several GB)
+        lines += int((d_in[s:min(nbytes, s + (1 << 28))] == 10).sum())
+    row = DS_ROW_BYTES + W
+    out = torch.empty(max(lines * row, DS_ROW_BYTES), dtype=torch.uint8, device=d_in.device)
+    stream = torch.cuda.current_stream(d_in.device)
+    tot = Totals()
+    rows = 0
+    if nbytes:
+        with Context(OP_DOSAGE, mode, device=d_in.device.index or 0, flags=F_DS_MATRIX, width=W, stream=stream.cuda_stream) as ctx:
+            if line_hint:
+                ctx.set_line_hint(line_hint)
+            ctx.run_device(d_in.data_ptr(), nbytes, out.data_ptr(), out.numel())
+            st = ctx.sync()
+        tot.add(st, 0, [])
+        rows = int(st.rows)
+    meta = out[:DS_ROW_BYTES * rows].view(rows, DS_ROW_BYTES)
+    return DosageMatrix(names, out[DS_ROW_BYTES * rows:DS_ROW_BYTES * rows + rows * W].view(torch.int8).view(rows, W),
+                        meta.view(torch.int64)[:, 0], meta.view(torch.int32)[:, 2], meta[:, 12].view(torch.bool),
+                        tot, DS_WARNING * tot.short_lines)
 
 
 F_GQ_STRICT = 1

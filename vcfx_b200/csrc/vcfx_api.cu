@@ -16,6 +16,8 @@
 
 using namespace vcfx;
 
+static_assert(sizeof(vcfx_ds_row) == 16, "ds_matrix_kernel writes a row's metadata as one 16-byte store");
+
 // kernel launches go through one macro so that the test-only warp emulator (tests/emu/) can build this file with g++
 #ifndef VCFX_LAUNCH
 #define VCFX_LAUNCH(kern, grid, block, smem, stream, arg) (kern)<<<(grid), (block), (smem), (stream)>>>(arg)
@@ -174,7 +176,9 @@ kernel_fn general_kernel_for(int op) {
     default: return nullptr;
     }
 }
-kernel_fn format_kernel_for(int op, int ac_fmt = 0) {
+bool is_ds_matrix(const vcfx_cfg &cfg) { return cfg.op == VCFX_OP_DOSAGE && (cfg.flags & VCFX_F_DS_MATRIX); }
+
+kernel_fn format_kernel_for(int op, int ac_fmt = 0, bool ds_matrix = false) {
     if (op == VCFX_OP_ALLELE_COUNT) return ac_fmt == AC_AGG ? format_rows_kernel<OP_AC> : nullptr;
     switch (op) {
     case VCFX_OP_ALLELE_FREQ: return format_rows_kernel<OP_AF>;
@@ -185,7 +189,7 @@ kernel_fn format_kernel_for(int op, int ac_fmt = 0) {
     case VCFX_OP_GENOTYPE_QUERY: return md_copy_kernel;
     case VCFX_OP_INDEX: return format_rows_kernel<OP_IX>;
     case VCFX_OP_INBREEDING: return ib_rows_kernel;
-    case VCFX_OP_DOSAGE: return ds_rows_kernel;
+    case VCFX_OP_DOSAGE: return ds_matrix ? ds_matrix_kernel : ds_rows_kernel;
     default: return nullptr;
     }
 }
@@ -388,6 +392,8 @@ int launch_chunk(vcfx_ctx *ctx, Work &w, cudaStream_t st, uint8_t *d_in, size_t 
     memcpy(P.gq_query, ctx->gq_query, sizeof P.gq_query); P.gq_len = ctx->gq_len; P.gq_a = ctx->gq_a; P.gq_b = ctx->gq_b; P.gq_strict = (ctx->cfg.flags & VCFX_F_GQ_STRICT) ? 1 : 0;
     P.ib_codes = w.ib_codes; P.ib_rows = w.ib_rows; P.ib_panels = w.ib_panels; P.ib_panel_cap = w.ib_panel_cap; P.ib = ctx->d_ib; P.ib_seq = w.ib_seq; P.ib_first = w.ib_first ? 1 : 0; P.text_cap = out_cap;
     if (ctx->cfg.op == VCFX_OP_INBREEDING) P.out_cap = ~0ULL;       // the scan counts rows there, not bytes of text
+    P.ds_matrix = is_ds_matrix(ctx->cfg) ? 1 : 0;
+    P.unit_bytes = P.ds_matrix ? 16u + (uint64_t)ctx->n_sel : 1u;   // matrix mode: rows x (16 + W) <= out_cap once the rows are counted
     P.stats = w.d_stats; P.events = w.events; P.ev_cap = w.ev_cap; P.ev_raw = (ctx->cfg.op == VCFX_OP_PHASE_CHECK || ctx->cfg.op == VCFX_OP_GENOTYPE_QUERY) ? 1 : 0;
 
     CU(cudaEventRecord(w.ev_k0, st));
@@ -402,7 +408,7 @@ int launch_chunk(vcfx_ctx *ctx, Work &w, cudaStream_t st, uint8_t *d_in, size_t 
         }
         VCFX_LAUNCH(tile_scan_kernel, 1, 1024, SCAN_SMEM_BYTES, st, P);
         CU(cudaGetLastError());
-        if (kernel_fn ff = format_kernel_for(ctx->cfg.op, ctx->ac_fmt)) {
+        if (kernel_fn ff = format_kernel_for(ctx->cfg.op, ctx->ac_fmt, is_ds_matrix(ctx->cfg))) {
             VCFX_LAUNCH(ff, ctx->sm_count * ((is_copy_op(ctx->cfg.op)) ? 8 : 16), 256, 0, st, P);
             CU(cudaGetLastError());
         } else if (ctx->cfg.op == VCFX_OP_ALLELE_COUNT) {
@@ -473,7 +479,10 @@ size_t default_out_bytes(int op, unsigned flags, size_t chunk) {
     case VCFX_OP_NONREF_FILTER: return chunk + 4096;          // never longer than the input plus one '\n'
     case VCFX_OP_PHASE_CHECK: return chunk + 4096;
     case VCFX_OP_GENOTYPE_QUERY: return chunk + 4096;
-    case VCFX_OP_DOSAGE: return chunk + 4096;                 // a sample column of two bytes or more gives at most two
+    case VCFX_OP_DOSAGE:
+        // text: a sample column of two bytes or more gives at most two.  Matrix: a row takes 16 + W bytes, no more than its
+        // line when the line has W columns of two bytes or more (W >= 7); rows of fewer columns grow the slot once
+        return chunk + 4096;
     case VCFX_OP_INBREEDING: return 1u << 20;                 // create() sizes it from the names
     case VCFX_OP_ALLELE_COUNT:
         if (flags & VCFX_F_AC_AGGREGATE) return chunk / 4 + (1u << 20);
@@ -637,6 +646,7 @@ int vcfx_cuda_create(const vcfx_cfg *cfg, vcfx_ctx **out) {
         CUC(cudaEventCreateWithFlags(&ctx->ib_event, cudaEventDisableTiming));
         if (!cfg->out_bytes) ctx->out_bytes = nb + (size_t)cfg->n_sel * 48 + 4096;      // "name \t F \n" per sample
     }
+    if (is_ds_matrix(*cfg)) ctx->n_sel = cfg->n_sel;               // W, the sample columns of the matrix (0 is valid)
     if (cfg->stream) { ctx->dev_stream = (cudaStream_t)cfg->stream; ctx->dev_stream_owned = false; }
     else { CUC(cudaStreamCreateWithFlags(&ctx->dev_stream, cudaStreamNonBlocking)); ctx->dev_stream_owned = true; }
 #undef CUC
@@ -903,6 +913,7 @@ int vcfx_cuda_short_lines(vcfx_ctx *ctx, uint64_t *line_no, size_t cap, size_t *
 int vcfx_cuda_run_device(vcfx_ctx *ctx, void *d_in, size_t nbytes, const vcfx_chunk_info *info,
                          void *d_out, size_t out_cap) {
     if (!ctx || !d_in || ((uintptr_t)d_in & 15)) return VCFX_E_INVALID;
+    if (is_ds_matrix(ctx->cfg) && ((uintptr_t)d_out & 15)) return VCFX_E_INVALID;     // the row metadata is written in 16-byte stores
     CU(cudaSetDevice(ctx->device));
     int rc = ensure_work(ctx, ctx->dev_work, nbytes);
     if (rc != VCFX_OK) return rc;

@@ -150,6 +150,9 @@ struct KParams {
     int32_t ib_first;                // first chunk of a stream: the per-sample state starts from zero
     uint64_t text_cap;               // bytes the final text may take in out (out_cap is not compared with the row count)
     int32_t ev_raw;                  // 1: events are final values (phase_checker: line offset << 2 | kind), not (tile, index) keys
+    // DOSAGE matrix mode (VCFX_F_DS_MATRIX): a row is one unit of tile output (tile_base + off_in_tile = its rank), n_sel = W
+    int32_t ds_matrix;
+    uint64_t unit_bytes;             // output bytes per unit of tile output: 1, or 16 + W in matrix mode (tile_scan_kernel's bytes_out)
 };
 
 // ---------------------------------------------------------------------------------------
@@ -2297,7 +2300,11 @@ __device__ __forceinline__ bool tile_lines(const KParams &P, const WarpShared ws
                                 P.recs[slot] = r;
                             }
                         }
-                        out_bytes += prefix_len + dlen + 1u; VCFX_COUNT(C_ROWS, 1);
+                        if (P.ds_matrix) {
+                            out_bytes += 1u;                             // matrix mode: the row's rank, not its text
+                            if (ncols > P.n_sel) VCFX_COUNT(C_FLAG, 1);  // columns beyond W are dropped
+                        } else out_bytes += prefix_len + dlen + 1u;
+                        VCFX_COUNT(C_ROWS, 1);
                     }
                 }
             }
@@ -2630,7 +2637,7 @@ tile_scan_kernel(const KParams P) {
         __syncthreads();
     }
     __syncthreads();
-    if (tid == 0) P.stats->bytes_out = carry_o;
+    if (tid == 0) P.stats->bytes_out = carry_o * P.unit_bytes;
     __syncthreads();
     unsigned long long nev = P.stats->n_events;
     if (nev > P.ev_cap) nev = P.ev_cap;
@@ -2997,6 +3004,76 @@ ds_rows_kernel(const KParams P) {
         __syncwarp();
         warp_flush_smem(o + flushed, stage + base, r.b + 1u - flushed, lane);
         __syncwarp();
+    }
+}
+
+// dosage_calculator matrix mode (VCFX_F_DS_MATRIX), K2b: a warp per row record.  The output is rows x 16 B of metadata
+// {uint64 line offset, uint32 columns, uint32 flags} followed by the rows x W int8 codes, row `rank` at 16 rows + rank W:
+// 0 / 1 / 2 the dosage, -1 "NA" (IB_NONE, IB_ABSENT, every column of a line without a GT key), -2 no such column.
+// A row is put together in shared memory at the destination's offset modulo 16, DSM_STEP samples at a time, and leaves in
+// aligned 128-bit stores; every lane builds 16 staged bytes from five aligned 32-bit loads of the codes.
+constexpr uint32_t DSM_STAGE = 2048, DSM_STEP = DSM_STAGE - 16;     // DSM_STEP is a multiple of 16: every step has the same phase
+__device__ __forceinline__ uint32_t ds_matrix_word(uint32_t q, int s0, uint32_t ncols, bool no_gt) {
+    const uint32_t na = ((q >> 2) | (q & (q >> 1))) & 0x01010101u;    // bytes holding IB_NONE (3) or IB_ABSENT (4)
+    const uint32_t v = q | (na * 0xFFu);
+    uint32_t w = 0;
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+        const int s = s0 + j;
+        const uint32_t b = (s >= (int)ncols) ? 0xFEu : (no_gt ? 0xFFu : ((v >> (8 * j)) & 0xFFu));
+        w |= b << (8 * j);
+    }
+    return w;
+}
+__global__ void __launch_bounds__(256)
+ds_matrix_kernel(const KParams P) {
+    __shared__ __align__(16) uint8_t s_stage[8][DSM_STAGE];
+    if (P.stats->overflow) return;
+    const int lane = threadIdx.x & 31;
+    uint8_t *stage = s_stage[threadIdx.x >> 5];
+    const uint32_t W = P.n_sel;
+    const unsigned long long rows = P.stats->rows;
+    uint8_t *const mat = P.out + 16ULL * rows;
+    const unsigned long long nrec = P.stats->n_recs;
+    const unsigned long long nwarps = (unsigned long long)gridDim.x * (blockDim.x >> 5);
+    for (unsigned long long i = (unsigned long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); i < nrec; i += nwarps) {
+        const Rec r = P.recs[i];
+        if (r.tile == REC_INVALID) continue;
+        const unsigned long long line = (unsigned long long)r.tile * P.tile_bytes + r.ls_rel;
+        const unsigned long long rank = P.tile_base[r.tile] + r.off_in_tile;
+        if (lane == 0) {
+            const unsigned long long off = P.file_offset + line;
+            *reinterpret_cast<uint4 *>(P.out + 16ULL * rank) = make_uint4((uint32_t)off, (uint32_t)(off >> 32), r.a, r.c);
+        }
+        if (W == 0) continue;
+        uint8_t *const dst = mat + rank * (unsigned long long)W;              // past 2^32 for realistic shapes
+        const uint8_t *const codes = P.ib_codes + ((line & ~3ULL) + r.d);
+        const uint32_t ncols = min(r.a, W);
+        const bool no_gt = r.c != 0;
+        const int base = (int)((uintptr_t)dst & 15u);
+        const int sh = (int)(((uintptr_t)codes - (uintptr_t)base) & 3u);    // staged byte k of a step holds sample f + k - base
+        for (uint32_t f = 0; f < W; f += DSM_STEP) {
+            const uint32_t n = min(W - f, DSM_STEP);
+            for (uint32_t k = 16u * (uint32_t)lane; k < (uint32_t)base + n; k += 512u) {
+                const int s0 = (int)(f + k) - base;                            // sample of staged byte k
+                const int t0 = s0 - sh;                                        // sample of the aligned word that holds it
+                uint32_t w[5];
+#pragma unroll
+                for (int j = 0; j < 5; ++j) {
+                    const int t = t0 + 4 * j;
+                    w[j] = (!no_gt && t + 3 >= 0 && t < (int)ncols) ? ldw(codes + t) : 0u;
+                }
+                uint4 o;
+                o.x = ds_matrix_word(__funnelshift_r(w[0], w[1], 8u * sh), s0, ncols, no_gt);
+                o.y = ds_matrix_word(__funnelshift_r(w[1], w[2], 8u * sh), s0 + 4, ncols, no_gt);
+                o.z = ds_matrix_word(__funnelshift_r(w[2], w[3], 8u * sh), s0 + 8, ncols, no_gt);
+                o.w = ds_matrix_word(__funnelshift_r(w[3], w[4], 8u * sh), s0 + 12, ncols, no_gt);
+                *reinterpret_cast<uint4 *>(stage + k) = o;
+            }
+            __syncwarp();
+            warp_flush_smem(dst + f, stage + base, n, lane);
+            __syncwarp();
+        }
     }
 }
 
