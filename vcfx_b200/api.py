@@ -354,14 +354,24 @@ import atexit  # noqa: E402
 atexit.register(close_cached_contexts)
 
 
-def _run(op: int, data: bytes, mode: int, chunk_bytes: int, flags: int = 0, device: int = 0, on_events=None, **kw):
-    # default slot size: the input rounded up to 1 MiB, at most 64 MiB (pinned allocations are not free)
+def _stream(op: int, data, mode: int, chunk_bytes: int, flags: int = 0, device: int = 0, valid_abs: int = 0, fmt0_abs: int = 0,
+            on_events=None, final_if_empty: bool = False, **kw):
+    """One stream of ``data`` through a context of ``op`` from _cached_context: (list of output pieces, Totals), as
+    stream_bytes.  The chunk size defaults to the input rounded up to 1 MiB, at most 64 MiB (pinned allocations are not
+    free).  On any exception the context leaves the cache and is closed: chunks of the failed stream may still be in
+    flight in it, and the next stream would drain them.  ``final_if_empty``: no bytes are still submitted, as one final
+    chunk (inbreeding_calculator reports with its final chunk)."""
     chunk_bytes = chunk_bytes or min(64 << 20, max(1 << 20, (len(data) + (1 << 20) - 1) & ~((1 << 20) - 1)))
     ctx, cached = _cached_context(op, mode, device, flags, chunk_bytes, **kw)
     try:
-        valid_abs = find_chrom_header(data) if op in (OP_ALLELE_FREQ, OP_NONREF_FILTER, OP_PHASE_CHECK) else 0
-        fmt0_abs = first_format_line(data, valid_abs) if (op == OP_PHASE_CHECK and mode == FILE) else 0
-        outs, tot = stream_bytes(ctx, data, chunk_bytes, valid_abs, on_events, fmt0_abs)
+        if len(data) == 0 and final_if_empty:
+            ctx.acquire()
+            ctx.submit(0, is_final=True)
+            out, st, _ = ctx.next_output()
+            tot = Totals(); tot.add(st, 0, [])
+            outs = [out]
+        else:
+            outs, tot = stream_bytes(ctx, data, chunk_bytes, valid_abs, on_events, fmt0_abs)
     except Exception:
         if cached:
             _ctx_cache.pop(next(k for k, v in _ctx_cache.items() if v is ctx), None)
@@ -369,6 +379,13 @@ def _run(op: int, data: bytes, mode: int, chunk_bytes: int, flags: int = 0, devi
         raise
     if not cached:
         ctx.close()
+    return outs, tot
+
+
+def _run(op: int, data: bytes, mode: int, chunk_bytes: int, **kw):
+    valid_abs = find_chrom_header(data) if op in (OP_ALLELE_FREQ, OP_NONREF_FILTER, OP_PHASE_CHECK) else 0
+    fmt0_abs = first_format_line(data, valid_abs) if (op == OP_PHASE_CHECK and mode == FILE) else 0
+    outs, tot = _stream(op, data, mode, chunk_bytes, valid_abs=valid_abs, fmt0_abs=fmt0_abs, **kw)
     return b"".join(outs), tot
 
 
@@ -427,9 +444,7 @@ def first_format_line(data, start: int = 0) -> int:
 
 
 def missing_detector(data: bytes, mode: int = FILE, chunk_bytes: int = 0, **kw) -> ToolResult:
-    chunk_bytes = chunk_bytes or min(64 << 20, max(1 << 20, (len(data) + (1 << 20) - 1) & ~((1 << 20) - 1)))
-    ctx, _ = _cached_context(OP_MISSING_DETECT, mode, 0, 0, chunk_bytes, **kw)
-    outs, tot = stream_bytes(ctx, data, chunk_bytes, first_data_offset(data))
+    outs, tot = _stream(OP_MISSING_DETECT, data, mode, chunk_bytes, valid_abs=first_data_offset(data), **kw)
     if mode == FILE and tot.last_unterminated_flagged and tot.dots_terminated == 0:
         # The reference's pre-scan ignores an unterminated last line (missing_detector.cpp:354): when
         # no other line has a '.' in its sample columns it copies the file verbatim, so that last
@@ -472,9 +487,7 @@ def indexer(data: bytes, mode: int = FILE, chunk_bytes: int = 0, **kw) -> ToolRe
     """VCFX_indexer: CHROM, POS and byte offset of every data line behind the "#CHROM" line.  totals.pre_header = 1 when
     the tool prints "Error: no #CHROM header found before variant lines."."""
     hdr_off, warned = _index_header(data, mode)
-    chunk_bytes = chunk_bytes or min(64 << 20, max(1 << 20, (len(data) + (1 << 20) - 1) & ~((1 << 20) - 1)))
-    ctx, cached = _cached_context(OP_INDEX, mode, 0, 0, chunk_bytes, **kw)
-    outs, tot = stream_bytes(ctx, data, chunk_bytes, hdr_off)
+    outs, tot = _stream(OP_INDEX, data, mode, chunk_bytes, valid_abs=hdr_off, **kw)
     tot.pre_header = int(warned)
     return ToolResult((INDEX_HEADER if hdr_off < len(data) else b"") + b"".join(outs), 0, tot)
 
@@ -538,26 +551,10 @@ def inbreeding_calculator(data: bytes, mode: int = FILE, freq_global: bool = Fal
     if mode == STDIN and not names:
         return ToolResult(IB_HEADER, 0, Totals(), IB_MESSAGES[5])
     flags = (F_IB_GLOBAL if freq_global else 0) | (F_IB_SKIP_BOUNDARY if skip_boundary else 0) | (F_IB_COUNT_BOUNDARY if count_boundary else 0)
-    body = data[start:]
-    chunk_bytes = chunk_bytes or min(64 << 20, max(1 << 20, (len(body) + (1 << 20) - 1) & ~((1 << 20) - 1)))
-    # (a context is good for one stream after the other: the per-sample state starts again behind a final chunk)
-    ctx, cached = _cached_context(OP_INBREEDING, mode, 0, flags, chunk_bytes, sel_cols=list(range(len(names))), sel_names=names, **kw)
-    try:
-        if len(body) == 0:                                 # no data line at all: a final chunk of nothing still reports
-            buf, cap = ctx.acquire()
-            ctx.submit(0, is_final=True)
-            out, st, _ = ctx.next_output()
-            tot = Totals(); tot.add(st, 0, [])
-            outs = [out]
-        else:
-            outs, tot = stream_bytes(ctx, body, chunk_bytes, 0)
-    except Exception:
-        if cached:
-            _ctx_cache.pop(next(k for k, v in _ctx_cache.items() if v is ctx), None)
-        ctx.close()
-        raise
-    if not cached:
-        ctx.close()
+    # (a context is good for one stream after the other: the per-sample state starts again behind a final chunk; with no
+    # data line at all, a final chunk of nothing still reports)
+    outs, tot = _stream(OP_INBREEDING, data[start:], mode, chunk_bytes, flags=flags, final_if_empty=True,
+                        sel_cols=list(range(len(names))), sel_names=names, **kw)
     err = IB_MESSAGES[3] if (tot.rows == 0 and not quiet) else b""
     return ToolResult(IB_HEADER + b"".join(outs), 0, tot, err)
 
@@ -648,15 +645,7 @@ def dosage_matrix(data: bytes, mode: int = FILE, width: int | None = None, chunk
     W = len(names) if width is None else int(width)
     metas, codes, tot = [], [], Totals()
     if len(data):
-        chunk_bytes = chunk_bytes or min(64 << 20, max(1 << 20, (len(data) + (1 << 20) - 1) & ~((1 << 20) - 1)))
-        ctx, cached = _cached_context(OP_DOSAGE, mode, 0, F_DS_MATRIX, chunk_bytes, width=W, **kw)
-        try:
-            outs, tot = stream_bytes(ctx, data, chunk_bytes)
-        except Exception:
-            if cached:
-                _ctx_cache.pop(next(k for k, v in _ctx_cache.items() if v is ctx), None)
-            ctx.close()
-            raise
+        outs, tot = _stream(OP_DOSAGE, data, mode, chunk_bytes, flags=F_DS_MATRIX, width=W, **kw)
         for piece in outs:
             m, c = _ds_split(piece, W)
             metas.append(m); codes.append(c)
@@ -758,17 +747,8 @@ def genotype_query(data: bytes, query: str, mode: int = FILE, strict: bool = Fal
 
     tot = Totals(); out = b""
     if body:
-        chunk_bytes = chunk_bytes or min(64 << 20, max(1 << 20, (len(body) + (1 << 20) - 1) & ~((1 << 20) - 1)))
-        ctx, cached = _cached_context(OP_GENOTYPE_QUERY, mode, 0, F_GQ_STRICT if strict else 0, chunk_bytes, query=q, **kw)
-        try:
-            outs, tot = stream_bytes(ctx, body, chunk_bytes, 0, on_events)
-        except Exception:
-            if cached:
-                _ctx_cache.pop(next(k for k, v in _ctx_cache.items() if v is ctx), None)
-            ctx.close()
-            raise
-        if not cached:
-            ctx.close()
+        outs, tot = _stream(OP_GENOTYPE_QUERY, body, mode, chunk_bytes, flags=F_GQ_STRICT if strict else 0, on_events=on_events,
+                            query=q, **kw)
         out = b"".join(outs)
     return ToolResult(out, 0, tot, b"" if quiet else b"".join(warn + msgs))
 

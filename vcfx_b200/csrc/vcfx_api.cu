@@ -29,6 +29,58 @@ constexpr size_t DEFAULT_CHUNK = 64u << 20;
 constexpr uint32_t EVENT_CAP = 1u << 20;
 constexpr int MAX_SLOTS = 8;
 
+typedef void (*kernel_fn)(const KParams);
+
+// What the host side needs to know about an operation, one row per vcfx_op (create() sets up the rest: allele_counter's
+// selection, genotype_query's query, inbreeding_calculator's per-sample state, the dosage matrix)
+struct OpInfo {
+    kernel_fn scan;
+    kernel_fn general;      // finishes the tiles the lattice kernel left (tile-resume array), or null
+    kernel_fn format;       // writes the rows from the row records, or null (no records)
+    bool copy;              // the output is the input with lines dropped or rewritten (md_copy_kernel): tail arrays, 8 CTAs per SM
+    bool raw_events;        // events are (offset << 2 | reason) words of dropped lines, and every one is kept (the list grows)
+    bool row_prefix;        // rows keep a 32-byte copy of their prefix
+    bool codes;             // the scan leaves a genotype code per sample column, one byte per input byte
+    bool reruns;            // a chunk may have to run again (more rows or text than sized for); a shared chunk is then copied
+    size_t (*out_bytes)(unsigned flags, size_t chunk);   // default output slot for chunks of `chunk` bytes
+};
+
+static_assert(VCFX_OP_VARIANT_COUNT == OP_VC && VCFX_OP_ALLELE_FREQ == OP_AF && VCFX_OP_HWE == OP_HWE && VCFX_OP_MISSING_DETECT == OP_MD &&
+              VCFX_OP_ALLELE_COUNT == OP_AC && VCFX_OP_NONREF_FILTER == OP_NR && VCFX_OP_INDEX == OP_IX && VCFX_OP_PHASE_CHECK == OP_PC &&
+              VCFX_OP_INBREEDING == OP_IB && VCFX_OP_GENOTYPE_QUERY == OP_GQ && VCFX_OP_DOSAGE == OP_DS, "OPS is indexed by vcfx_op");
+constexpr OpInfo OPS[] = {
+    //  scan                        general                     format                       copy   raw    prefix codes  reruns
+    {vcfx_scan_kernel<OP_VC, 0>,  nullptr,                    nullptr,                     false, false, false, false, false,
+     [](unsigned, size_t) -> size_t { return 4096; }},
+    {vcfx_scan_kernel<OP_AF, 0>,  vcfx_scan_kernel<OP_AF, 1>,  format_rows_kernel<OP_AF>,   false, false, true,  false, true,
+     [](unsigned, size_t c) -> size_t { return c / 4 + (1u << 20); }},          // rows are ~0.3 % of the input
+    {vcfx_scan_kernel<OP_HWE, 0>, vcfx_scan_kernel<OP_HWE, 1>, format_rows_kernel<OP_HWE>,  false, false, true,  false, true,
+     [](unsigned, size_t c) -> size_t { return c / 4 + (1u << 20); }},
+    {vcfx_scan_kernel<OP_MD, 0>,  nullptr,                    md_copy_kernel,              true,  false, false, false, true,
+     [](unsigned, size_t c) -> size_t { return c + c / 4 + 4096; }},
+    {vcfx_scan_kernel<OP_AC, 0>,  nullptr,                    format_rows_kernel<OP_AC>,   false, false, false, false, true,
+     [](unsigned flags, size_t c) -> size_t {
+         if (flags & VCFX_F_AC_AGGREGATE) return c / 4 + (1u << 20);
+         if (flags & VCFX_F_AC_BINARY) return c + 4096;
+         return 10 * c + 4096;                                                  // a text row per genotype: ~9x the input at 2,504 samples
+     }},
+    {vcfx_scan_kernel<OP_NR, 0>,  nullptr,                    md_copy_kernel,              true,  false, false, false, true,
+     [](unsigned, size_t c) -> size_t { return c + 4096; }},                    // never longer than the input plus one '\n'
+    {vcfx_scan_kernel<OP_IX, 0>,  nullptr,                    format_rows_kernel<OP_IX>,   false, false, false, false, true,
+     [](unsigned, size_t c) -> size_t { return c / 4 + (1u << 20); }},
+    {vcfx_scan_kernel<OP_PC, 0>,  nullptr,                    md_copy_kernel,              true,  true,  false, false, true,
+     [](unsigned, size_t c) -> size_t { return c + 4096; }},
+    {vcfx_scan_kernel<OP_IB, 0>,  nullptr,                    ib_rows_kernel,              false, false, false, true,  true,
+     [](unsigned, size_t) -> size_t { return 1u << 20; }},                      // create() sizes it from the names
+    {vcfx_scan_kernel<OP_GQ, 0>,  nullptr,                    md_copy_kernel,              true,  true,  false, false, true,
+     [](unsigned, size_t c) -> size_t { return c + 4096; }},
+    // text: a sample column of two bytes or more gives at most two.  Matrix: a row takes 16 + W bytes, no more than its line
+    // when the line has W columns of two bytes or more (W >= 7); rows of fewer columns grow the slot once
+    {vcfx_scan_kernel<OP_DS, 0>,  nullptr,                    ds_rows_kernel,              false, false, false, true,  true,
+     [](unsigned, size_t c) -> size_t { return c + 4096; }},
+};
+constexpr int N_OPS = (int)(sizeof OPS / sizeof OPS[0]);
+
 struct Work {                      // device-side bookkeeping for one launch
     uint32_t *tile_lines = nullptr;
     unsigned long long *tile_out = nullptr;
@@ -79,6 +131,10 @@ struct Slot {
 
 struct vcfx_ctx {
     vcfx_cfg cfg;
+    const OpInfo *op = nullptr;          // OPS[cfg.op]
+    kernel_fn format = nullptr;          // the row writer launched behind the scan (op->format, or allele_counter's / the matrix's)
+    bool two_pass = false;               // allele_counter text / binary: rows are sized in a first scan and written in a second
+    bool ds_matrix = false;              // dosage_calculator with VCFX_F_DS_MATRIX
     int device = 0;
     int sm_count = 0;
     int blocks_per_sm = 1;
@@ -101,7 +157,7 @@ struct vcfx_ctx {
     uint8_t *dev_in = nullptr, *dev_out = nullptr;
     size_t dev_out_cap = 0;
     vcfx_chunk_info dev_info = {0, 1, 0, 0};
-    // allele_counter selection (device copies)
+    // allele_counter selection (device copies); max_col = 0 for the other ops (no column scratch)
     uint32_t n_sel = 0, max_col = 0;
     uint32_t *d_sel_col = nullptr, *d_name_off = nullptr;
     uint8_t *d_names = nullptr;
@@ -110,11 +166,12 @@ struct vcfx_ctx {
     bool ac_bulk = true;                 // staged rows leave shared memory through cp.async.bulk (VCFX_AC_BULK=0: 128-bit stores)
     int ac_fmt = 0;
     bool ac_ident = false;               // allele_counter selection = columns 0 .. n_sel-1 in order
-    bool ac_exact = false;               // a chunk had a count of two digits: rows are sized by parsing from now on
+    bool ac_spec = false;                // allele_counter text: rows are sized by speculation until a chunk has a count of two digits
     bool c4_bulk = false;                // VCFX_C4_BULK=1: the skip-ahead loop reads through the bulk-copy ring (see vcfx_kernels.cuh)
     // genotype_query: the query and what parseDiploidAlleles leaves of it
     uint8_t gq_query[64] = {0}; uint32_t gq_len = 0; int gq_a = -1, gq_b = -1;
-    // inbreeding_calculator: the per-sample state that lives from chunk to chunk, and the order the chunks are applied in
+    // inbreeding_calculator (d_ib is null for the other ops): the per-sample state that lives from chunk to chunk, and the
+    // order the chunks are applied in
     IbState *d_ib = nullptr; double *d_ib_sum = nullptr; unsigned long long *d_ib_het = nullptr; unsigned int *d_ib_used = nullptr; uint8_t *d_ib_last = nullptr;
     cudaEvent_t ib_event = nullptr;      // the last chunk launched has been applied
     bool ib_event_set = false;
@@ -137,8 +194,6 @@ namespace {
         }                                                                                \
     } while (0)
 
-typedef void (*kernel_fn)(const KParams);
-
 #ifdef VCFX_EMU
 struct HweArgs { const int32_t *c; size_t n; double *p; };
 void hwe_pvalue_entry(const HweArgs a) { hwe_pvalue_kernel(a.c, a.n, a.p); }
@@ -146,53 +201,6 @@ void hwe_pvalue_launch(int grid, const int32_t *c, size_t n, double *p) { HweArg
 #else
 void hwe_pvalue_launch(int grid, const int32_t *c, size_t n, double *p) { hwe_pvalue_kernel<<<grid, 256>>>(c, n, p); }
 #endif
-
-// ops whose output is the input with lines dropped or rewritten (md_copy_kernel writes it)
-bool is_copy_op(int op) {
-    return op == VCFX_OP_MISSING_DETECT || op == VCFX_OP_NONREF_FILTER || op == VCFX_OP_PHASE_CHECK || op == VCFX_OP_GENOTYPE_QUERY;
-}
-
-kernel_fn kernel_for(int op) {
-    switch (op) {
-    case VCFX_OP_VARIANT_COUNT: return vcfx_scan_kernel<OP_VC, 0>;
-    case VCFX_OP_ALLELE_FREQ:   return vcfx_scan_kernel<OP_AF, 0>;
-    case VCFX_OP_HWE:           return vcfx_scan_kernel<OP_HWE, 0>;
-    case VCFX_OP_MISSING_DETECT: return vcfx_scan_kernel<OP_MD, 0>;
-    case VCFX_OP_NONREF_FILTER: return vcfx_scan_kernel<OP_NR, 0>;
-    case VCFX_OP_INDEX: return vcfx_scan_kernel<OP_IX, 0>;
-    case VCFX_OP_PHASE_CHECK: return vcfx_scan_kernel<OP_PC, 0>;
-    case VCFX_OP_INBREEDING: return vcfx_scan_kernel<OP_IB, 0>;
-    case VCFX_OP_GENOTYPE_QUERY: return vcfx_scan_kernel<OP_GQ, 0>;
-    case VCFX_OP_DOSAGE: return vcfx_scan_kernel<OP_DS, 0>;
-    case VCFX_OP_ALLELE_COUNT:  return vcfx_scan_kernel<OP_AC, 0>;
-    default: return nullptr;
-    }
-}
-// the general kernel that finishes the tiles the lattice kernel left (allele_freq_calc / hwe_tester)
-kernel_fn general_kernel_for(int op) {
-    switch (op) {
-    case VCFX_OP_ALLELE_FREQ: return vcfx_scan_kernel<OP_AF, 1>;
-    case VCFX_OP_HWE:         return vcfx_scan_kernel<OP_HWE, 1>;
-    default: return nullptr;
-    }
-}
-bool is_ds_matrix(const vcfx_cfg &cfg) { return cfg.op == VCFX_OP_DOSAGE && (cfg.flags & VCFX_F_DS_MATRIX); }
-
-kernel_fn format_kernel_for(int op, int ac_fmt = 0, bool ds_matrix = false) {
-    if (op == VCFX_OP_ALLELE_COUNT) return ac_fmt == AC_AGG ? format_rows_kernel<OP_AC> : nullptr;
-    switch (op) {
-    case VCFX_OP_ALLELE_FREQ: return format_rows_kernel<OP_AF>;
-    case VCFX_OP_HWE:         return format_rows_kernel<OP_HWE>;
-    case VCFX_OP_MISSING_DETECT: return md_copy_kernel;
-    case VCFX_OP_NONREF_FILTER: return md_copy_kernel;
-    case VCFX_OP_PHASE_CHECK: return md_copy_kernel;
-    case VCFX_OP_GENOTYPE_QUERY: return md_copy_kernel;
-    case VCFX_OP_INDEX: return format_rows_kernel<OP_IX>;
-    case VCFX_OP_INBREEDING: return ib_rows_kernel;
-    case VCFX_OP_DOSAGE: return ds_matrix ? ds_matrix_kernel : ds_rows_kernel;
-    default: return nullptr;
-    }
-}
 
 // Bytes of input owned by one warp.  Larger tiles waste less on the overlap at tile borders (the
 // owner of a tile reads on to the end of its last line, and the next owner scans the same bytes for
@@ -292,11 +300,11 @@ int ensure_work(vcfx_ctx *ctx, Work &w, size_t max_bytes, uint64_t min_recs = 0,
         CU(cudaMalloc(&w.tile_out, sizeof(unsigned long long) * tiles));
         CU(cudaMalloc(&w.tile_base, sizeof(unsigned long long) * tiles));
         CU(cudaMalloc(&w.line_base, sizeof(unsigned long long) * tiles));
-        if (general_kernel_for(ctx->cfg.op)) {
+        if (ctx->op->general) {
             cudaFree(w.tile_resume); w.tile_resume = nullptr;
             CU(cudaMalloc(&w.tile_resume, sizeof(uint32_t) * tiles));
         }
-        if (is_copy_op(ctx->cfg.op)) {
+        if (ctx->op->copy) {
             cudaFree(w.tail_start); cudaFree(w.tail_len); cudaFree(w.tail_off);
             w.tail_start = w.tail_len = w.tail_off = nullptr;
             CU(cudaMalloc(&w.tail_start, sizeof(uint32_t) * tiles));
@@ -306,17 +314,17 @@ int ensure_work(vcfx_ctx *ctx, Work &w, size_t max_bytes, uint64_t min_recs = 0,
         w.tiles_cap = tiles;
     }
     uint64_t recs = 0;
-    if (format_kernel_for(ctx->cfg.op, ctx->ac_fmt)) recs = std::max<uint64_t>(default_rec_cap(max_bytes), min_recs);
-    if (ctx->cfg.op == VCFX_OP_ALLELE_COUNT && !w.col_scratch) {
+    if (ctx->format) recs = std::max<uint64_t>(default_rec_cap(max_bytes), min_recs);
+    if (ctx->max_col && !w.col_scratch) {
         size_t n = (size_t)ctx->sm_count * ctx->blocks_per_sm * WARPS_PER_CTA * std::max<uint32_t>(ctx->max_col, 1);
         CU(cudaMalloc(&w.col_scratch, n * sizeof(uint2)));
     }
-    if (ctx->cfg.op == VCFX_OP_DOSAGE && max_bytes + VCFX_DEVICE_PAD > w.ib_codes_cap) {      // a code per sample column, as for inbreeding_calculator
+    if (ctx->op->codes && max_bytes + VCFX_DEVICE_PAD > w.ib_codes_cap) {
         cudaFree(w.ib_codes); w.ib_codes = nullptr; w.ib_codes_cap = 0;
         CU(cudaMalloc(&w.ib_codes, max_bytes + VCFX_DEVICE_PAD));
         w.ib_codes_cap = max_bytes + VCFX_DEVICE_PAD;
     }
-    if (ctx->cfg.op == VCFX_OP_INBREEDING) {
+    if (ctx->d_ib) {
         // the codes once more in file order, 32 samples to a panel: lines that have all their columns need less than the
         // input has bytes; min_panel_bytes is what a chunk that did not fit asked for
         const uint64_t want_pan = std::max<uint64_t>(max_bytes + (1u << 20), min_panel_bytes);
@@ -324,11 +332,6 @@ int ensure_work(vcfx_ctx *ctx, Work &w, size_t max_bytes, uint64_t min_recs = 0,
             cudaFree(w.ib_panels); w.ib_panels = nullptr; w.ib_panel_cap = 0;
             CU(cudaMalloc(&w.ib_panels, want_pan));
             w.ib_panel_cap = want_pan;
-        }
-        if (max_bytes + VCFX_DEVICE_PAD > w.ib_codes_cap) {
-            cudaFree(w.ib_codes); w.ib_codes = nullptr; w.ib_codes_cap = 0;
-            CU(cudaMalloc(&w.ib_codes, max_bytes + VCFX_DEVICE_PAD));
-            w.ib_codes_cap = max_bytes + VCFX_DEVICE_PAD;
         }
         if (std::max<uint64_t>(recs, w.rec_cap) > w.ib_rows_cap) {
             const uint64_t want = std::max<uint64_t>(recs, w.rec_cap);
@@ -341,7 +344,7 @@ int ensure_work(vcfx_ctx *ctx, Work &w, size_t max_bytes, uint64_t min_recs = 0,
         cudaFree(w.recs); w.recs = nullptr; w.rec_cap = 0;
         cudaFree(w.rec_prefix); w.rec_prefix = nullptr;
         CU(cudaMalloc(&w.recs, recs * sizeof(Rec)));
-        if (ctx->cfg.op == VCFX_OP_ALLELE_FREQ || ctx->cfg.op == VCFX_OP_HWE) CU(cudaMalloc(&w.rec_prefix, recs * 32));
+        if (ctx->op->row_prefix) CU(cudaMalloc(&w.rec_prefix, recs * 32));
         w.rec_cap = recs;
     }
     return VCFX_OK;
@@ -355,7 +358,7 @@ uint64_t ib_panel_need(const vcfx_ctx *ctx, const Work &w) {
 // inbreeding_calculator: a NEW chunk takes the next place in the order its context applies chunks in (a chunk that is run
 // again keeps its place); the first chunk behind a final one starts a new stream
 void ib_begin(vcfx_ctx *ctx, Work &w, const vcfx_chunk_info *info) {
-    if (ctx->cfg.op != VCFX_OP_INBREEDING) return;
+    if (!ctx->d_ib) return;
     w.ib_seq = ctx->ib_next_seq++;
     w.ib_first = !ctx->ib_open;
     ctx->ib_open = !(info ? info->is_final != 0 : true);
@@ -364,14 +367,12 @@ void ib_begin(vcfx_ctx *ctx, Work &w, const vcfx_chunk_info *info) {
 // enqueue the kernels of one chunk on `st`; results land in w.h_stats after the stream drains
 int launch_chunk(vcfx_ctx *ctx, Work &w, cudaStream_t st, uint8_t *d_in, size_t nbytes,
                  const vcfx_chunk_info *info, uint8_t *d_out, size_t out_cap, bool write_pad = true) {
-    kernel_fn fn = kernel_for(ctx->cfg.op);
-    if (!fn) return VCFX_E_UNSUPPORTED;
+    const OpInfo &op = *ctx->op;
     const uint32_t tile = tile_for(ctx, nbytes);
     uint32_t tiles = tiles_for(ctx, nbytes, tile);
     if (write_pad) CU(cudaMemsetAsync(d_in + nbytes, '\n', 64, st));
     CU(cudaMemsetAsync(w.ticket, 0, 2 * sizeof(unsigned int), st));
-    kernel_fn gfn = general_kernel_for(ctx->cfg.op);
-    if (gfn) CU(cudaMemsetAsync(w.tile_resume, 0xFF, sizeof(uint32_t) * tiles, st));
+    if (op.general) CU(cudaMemsetAsync(w.tile_resume, 0xFF, sizeof(uint32_t) * tiles, st));
     CU(cudaMemcpyAsync(w.d_stats, w.h_init, sizeof(DevStats), cudaMemcpyHostToDevice, st));
 
     KParams P;
@@ -385,41 +386,41 @@ int launch_chunk(vcfx_ctx *ctx, Work &w, cudaStream_t st, uint8_t *d_in, size_t 
     P.out = d_out; P.out_cap = out_cap;
     P.tile_lines = w.tile_lines; P.tile_out = w.tile_out; P.tile_base = w.tile_base; P.line_base = w.line_base;
     P.tail_start = w.tail_start; P.tail_len = w.tail_len; P.tail_off = w.tail_off;
-    P.ac_fmt = ctx->ac_fmt; P.ac_ident = ctx->ac_ident ? 1 : 0; P.ac_pass = 0; P.ac_spec = (ctx->cfg.op == VCFX_OP_ALLELE_COUNT && ctx->ac_fmt == AC_TEXT_MT && !ctx->ac_exact) ? 1 : 0; P.n_sel = ctx->n_sel; P.sel_col = ctx->d_sel_col; P.name_off = ctx->d_name_off;
+    P.ac_fmt = ctx->ac_fmt; P.ac_ident = ctx->ac_ident ? 1 : 0; P.ac_pass = 0; P.ac_spec = ctx->ac_spec ? 1 : 0; P.n_sel = ctx->n_sel; P.sel_col = ctx->d_sel_col; P.name_off = ctx->d_name_off;
     P.names = ctx->d_names; P.names16 = ctx->d_names16; P.name_len = ctx->name_len; P.ac_bulk = ctx->ac_bulk ? 1 : 0; P.max_col = ctx->max_col; P.col_scratch = w.col_scratch;
     P.ticket = w.ticket; P.ticket2 = w.ticket + 1; P.tile_resume = w.tile_resume; P.recs = w.recs; P.rec_prefix = w.rec_prefix; P.rec_cap = w.rec_cap;
     P.c4_bulk = ctx->c4_bulk ? 1 : 0;
     memcpy(P.gq_query, ctx->gq_query, sizeof P.gq_query); P.gq_len = ctx->gq_len; P.gq_a = ctx->gq_a; P.gq_b = ctx->gq_b; P.gq_strict = (ctx->cfg.flags & VCFX_F_GQ_STRICT) ? 1 : 0;
     P.ib_codes = w.ib_codes; P.ib_rows = w.ib_rows; P.ib_panels = w.ib_panels; P.ib_panel_cap = w.ib_panel_cap; P.ib = ctx->d_ib; P.ib_seq = w.ib_seq; P.ib_first = w.ib_first ? 1 : 0; P.text_cap = out_cap;
-    if (ctx->cfg.op == VCFX_OP_INBREEDING) P.out_cap = ~0ULL;       // the scan counts rows there, not bytes of text
-    P.ds_matrix = is_ds_matrix(ctx->cfg) ? 1 : 0;
+    if (ctx->d_ib) P.out_cap = ~0ULL;       // the scan counts rows there, not bytes of text
+    P.ds_matrix = ctx->ds_matrix ? 1 : 0;
     P.unit_bytes = P.ds_matrix ? 16u + (uint64_t)ctx->n_sel : 1u;   // matrix mode: rows x (16 + W) <= out_cap once the rows are counted
-    P.stats = w.d_stats; P.events = w.events; P.ev_cap = w.ev_cap; P.ev_raw = (ctx->cfg.op == VCFX_OP_PHASE_CHECK || ctx->cfg.op == VCFX_OP_GENOTYPE_QUERY) ? 1 : 0;
+    P.stats = w.d_stats; P.events = w.events; P.ev_cap = w.ev_cap; P.ev_raw = op.raw_events ? 1 : 0;
 
     CU(cudaEventRecord(w.ev_k0, st));
     if (nbytes > 0) {
         int grid = grid_for(ctx, tiles);
-        VCFX_LAUNCH(fn, grid, WARPS_PER_CTA * 32, 0, st, P);
+        VCFX_LAUNCH(op.scan, grid, WARPS_PER_CTA * 32, 0, st, P);
         CU(cudaGetLastError());
-        if (gfn) {                       // finishes the tiles the lattice kernel left; exits at once when there are none
-            const int ggrid = std::max(1, std::min(ctx->sm_count * VCFX_GENERAL_CTAS, (int)((tiles + WARPS_PER_CTA - 1) / WARPS_PER_CTA)));
-            VCFX_LAUNCH(gfn, ggrid, WARPS_PER_CTA * 32, 0, st, P);
+        if (op.general) {                // finishes the tiles the lattice kernel left; exits at once when there are none
+            const int ggrid = std::max(1, std::min(ctx->sm_count * scan_ctas(ctx->cfg.op, 1), (int)((tiles + WARPS_PER_CTA - 1) / WARPS_PER_CTA)));
+            VCFX_LAUNCH(op.general, ggrid, WARPS_PER_CTA * 32, 0, st, P);
             CU(cudaGetLastError());
         }
         VCFX_LAUNCH(tile_scan_kernel, 1, 1024, SCAN_SMEM_BYTES, st, P);
         CU(cudaGetLastError());
-        if (kernel_fn ff = format_kernel_for(ctx->cfg.op, ctx->ac_fmt, is_ds_matrix(ctx->cfg))) {
-            VCFX_LAUNCH(ff, ctx->sm_count * ((is_copy_op(ctx->cfg.op)) ? 8 : 16), 256, 0, st, P);
+        if (ctx->format) {
+            VCFX_LAUNCH(ctx->format, ctx->sm_count * (op.copy ? 8 : 16), 256, 0, st, P);
             CU(cudaGetLastError());
-        } else if (ctx->cfg.op == VCFX_OP_ALLELE_COUNT) {
+        } else if (ctx->two_pass) {
             // rows are sized in the first pass and written in a second one at their scanned offsets
             CU(cudaMemsetAsync(w.ticket, 0, 2 * sizeof(unsigned int), st));
             P.ac_pass = 1;
-            VCFX_LAUNCH(fn, grid, WARPS_PER_CTA * 32, 0, st, P);
+            VCFX_LAUNCH(op.scan, grid, WARPS_PER_CTA * 32, 0, st, P);
             CU(cudaGetLastError());
         }
     }
-    if (ctx->cfg.op == VCFX_OP_INBREEDING) {
+    if (ctx->d_ib) {
         // the sample-axis pass: chunks are applied one after the other, whatever stream they were scanned on
         if (ctx->ib_event_set) CU(cudaStreamWaitEvent(st, ctx->ib_event, 0));
         VCFX_LAUNCH(ib_accumulate_kernel, (int)((ctx->n_sel + 31) / 32), 32, 0, st, P);   // (an empty chunk still opens or closes a stream)
@@ -460,36 +461,16 @@ int fetch_events(vcfx_ctx *ctx, const Work &w, cudaStream_t st) {
     return VCFX_OK;
 }
 
-// phase_checker reports every dropped line: a chunk that dropped more lines than the list holds gets a longer list (and
-// is run again by the caller).  Returns 1 when it grew, 0 when nothing was lost, a negative vcfx_err on failure.
+// phase_checker and genotype_query report every dropped line: a chunk that dropped more lines than the list holds gets a
+// longer list (and is run again).  Returns 1 when it grew, 0 when nothing was lost, a negative vcfx_err on failure.
 int grow_events(vcfx_ctx *ctx, Work &w) {
-    if ((ctx->cfg.op != VCFX_OP_PHASE_CHECK && ctx->cfg.op != VCFX_OP_GENOTYPE_QUERY) || w.h_stats->n_events <= w.ev_cap) return 0;
+    if (!ctx->op->raw_events || w.h_stats->n_events <= w.ev_cap) return 0;
     const uint64_t want = w.h_stats->n_events + (w.h_stats->n_events >> 3) + 1024;
     if (want > 0xFFFFFFFFull) return VCFX_E_OUTPUT_TOO_BIG;
     cudaFree(w.events); w.events = nullptr; w.ev_cap = 0;
     CU(cudaMalloc(&w.events, sizeof(unsigned long long) * want));
     w.ev_cap = (uint32_t)want;
     return 1;
-}
-
-size_t default_out_bytes(int op, unsigned flags, size_t chunk) {
-    switch (op) {
-    case VCFX_OP_VARIANT_COUNT: return 4096;
-    case VCFX_OP_MISSING_DETECT: return chunk + chunk / 4 + 4096;
-    case VCFX_OP_NONREF_FILTER: return chunk + 4096;          // never longer than the input plus one '\n'
-    case VCFX_OP_PHASE_CHECK: return chunk + 4096;
-    case VCFX_OP_GENOTYPE_QUERY: return chunk + 4096;
-    case VCFX_OP_DOSAGE:
-        // text: a sample column of two bytes or more gives at most two.  Matrix: a row takes 16 + W bytes, no more than its
-        // line when the line has W columns of two bytes or more (W >= 7); rows of fewer columns grow the slot once
-        return chunk + 4096;
-    case VCFX_OP_INBREEDING: return 1u << 20;                 // create() sizes it from the names
-    case VCFX_OP_ALLELE_COUNT:
-        if (flags & VCFX_F_AC_AGGREGATE) return chunk / 4 + (1u << 20);
-        if (flags & VCFX_F_AC_BINARY) return chunk + 4096;
-        return 10 * chunk + 4096;                // a text row per genotype: ~9x the input at 2,504 samples
-    default: return chunk / 4 + (1u << 20);      // AF / HWE rows are ~0.3 % of the input
-    }
 }
 
 // The text of finished chunks starts its way to the host as soon as their kernels are done, oldest first, whenever the
@@ -539,19 +520,20 @@ const char *vcfx_cuda_last_error(const vcfx_ctx *ctx) { return ctx ? ctx->last_e
 int vcfx_cuda_create(const vcfx_cfg *cfg, vcfx_ctx **out) {
     if (!cfg || !out) return VCFX_E_INVALID;
     *out = nullptr;
-    if (cfg->op < VCFX_OP_VARIANT_COUNT || cfg->op > VCFX_OP_DOSAGE) return VCFX_E_INVALID;
+    if (cfg->op < 0 || cfg->op >= N_OPS) return VCFX_E_INVALID;
     if (cfg->mode != VCFX_MODE_FILE && cfg->mode != VCFX_MODE_STDIN) return VCFX_E_INVALID;
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) return VCFX_E_NO_DEVICE;
     if (cfg->device < 0 || cfg->device >= ndev) return VCFX_E_INVALID;
-    if (!kernel_for(cfg->op)) return VCFX_E_UNSUPPORTED;
     vcfx_ctx *ctx = new (std::nothrow) vcfx_ctx();
     if (!ctx) return VCFX_E_NOMEM;
     ctx->cfg = *cfg;
+    ctx->op = &OPS[cfg->op];
+    ctx->format = ctx->op->format;
     ctx->device = cfg->device;
     ctx->chunk_bytes = cfg->chunk_bytes ? cfg->chunk_bytes : DEFAULT_CHUNK;
     ctx->tile_bytes = cfg->tile_bytes > 0 ? std::max<uint32_t>(512, ((uint32_t)cfg->tile_bytes + 511) & ~511u) : 0;   // 0 = per launch
-    ctx->out_bytes = cfg->out_bytes ? cfg->out_bytes : default_out_bytes(cfg->op, cfg->flags, ctx->chunk_bytes);
+    ctx->out_bytes = cfg->out_bytes ? cfg->out_bytes : ctx->op->out_bytes(cfg->flags, ctx->chunk_bytes);
     ctx->n_slots = cfg->n_slots > 0 ? std::min(cfg->n_slots, MAX_SLOTS) : 3;
     auto fail = [&](int rc) { std::string e = ctx->last_error; vcfx_cuda_destroy(ctx); (void)e; return rc; };
 #define CUC(call)                                                                        \
@@ -568,13 +550,15 @@ int vcfx_cuda_create(const vcfx_cfg *cfg, vcfx_ctx **out) {
     ctx->sm_count = prop.multiProcessorCount;
     int bps = 1;
     CUC(cudaFuncSetAttribute(tile_scan_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SCAN_SMEM_BYTES));
-    CUC(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, kernel_for(cfg->op), WARPS_PER_CTA * 32, 0));
+    CUC(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, ctx->op->scan, WARPS_PER_CTA * 32, 0));
     // the kernels are tuned at their __launch_bounds__ occupancy (variant_counter measured slower at 6 CTAs than at 5)
-    ctx->blocks_per_sm = std::max(1, std::min(bps, cfg->op == VCFX_OP_VARIANT_COUNT ? 5 : (cfg->op == VCFX_OP_ALLELE_COUNT ? VCFX_AC_CTAS : VCFX_PARSE_CTAS)));
+    ctx->blocks_per_sm = std::max(1, std::min(bps, scan_ctas(cfg->op, 0)));
     if (cfg->op == VCFX_OP_ALLELE_COUNT) {
         if (cfg->n_sel == 0 || !cfg->sel_col || !cfg->sel_names || !cfg->sel_name_off) return fail(VCFX_E_INVALID);
         ctx->ac_fmt = (cfg->flags & VCFX_F_AC_AGGREGATE) ? AC_AGG : (cfg->flags & VCFX_F_AC_BINARY) ? AC_BIN
                     : (cfg->flags & VCFX_F_AC_FORWARD) ? AC_TEXT_FWD : AC_TEXT_MT;
+        if (ctx->ac_fmt != AC_AGG) { ctx->format = nullptr; ctx->two_pass = true; }
+        ctx->ac_spec = ctx->ac_fmt == AC_TEXT_MT;
         std::vector<uint32_t> cols(cfg->sel_col, cfg->sel_col + cfg->n_sel);
         if (ctx->ac_fmt != AC_TEXT_MT)                      // forward-only column walk (:1222-1227): running maximum
             for (size_t i = 1; i < cols.size(); ++i) cols[i] = std::max(cols[i], cols[i - 1]);
@@ -646,7 +630,11 @@ int vcfx_cuda_create(const vcfx_cfg *cfg, vcfx_ctx **out) {
         CUC(cudaEventCreateWithFlags(&ctx->ib_event, cudaEventDisableTiming));
         if (!cfg->out_bytes) ctx->out_bytes = nb + (size_t)cfg->n_sel * 48 + 4096;      // "name \t F \n" per sample
     }
-    if (is_ds_matrix(*cfg)) ctx->n_sel = cfg->n_sel;               // W, the sample columns of the matrix (0 is valid)
+    if (cfg->op == VCFX_OP_DOSAGE && (cfg->flags & VCFX_F_DS_MATRIX)) {
+        ctx->ds_matrix = true;
+        ctx->format = ds_matrix_kernel;
+        ctx->n_sel = cfg->n_sel;                                    // W, the sample columns of the matrix (0 is valid)
+    }
     if (cfg->stream) { ctx->dev_stream = (cudaStream_t)cfg->stream; ctx->dev_stream_owned = false; }
     else { CUC(cudaStreamCreateWithFlags(&ctx->dev_stream, cudaStreamNonBlocking)); ctx->dev_stream_owned = true; }
 #undef CUC
@@ -744,6 +732,55 @@ static int ensure_slot(vcfx_ctx *ctx, Slot &s) {
     return ensure_work(ctx, s.w, ctx->chunk_bytes);
 }
 
+// What every submit ends with: the chunk in slot s, its bytes at d_in, is launched on the slot's stream and joins the
+// pipeline behind the chunks already in flight.
+static int start_chunk(vcfx_ctx *ctx, Slot &s, uint8_t *d_in, size_t nbytes, const vcfx_chunk_info *info) {
+    s.info = info ? *info : vcfx_chunk_info{0, 1, 0, 0, 0};
+    s.d_in_used = d_in;
+    ib_begin(ctx, s.w, &s.info);
+    int rc = launch_chunk(ctx, s.w, s.stream, d_in, nbytes, &s.info, s.d_out, s.out_cap, false);
+    if (rc != VCFX_OK) return rc;
+    s.nbytes = nbytes; s.in_flight = true; s.d2h_issued = false;
+    ctx->head = (ctx->head + 1) % ctx->n_slots;
+    ctx->n_in_flight++;
+    return VCFX_OK;
+}
+
+// the chunk's bytes go from host memory (the slot's pinned buffer, or the caller's) to the slot's device input, then start
+static int upload_and_start(vcfx_ctx *ctx, Slot &s, const void *host, size_t nbytes, const vcfx_chunk_info *info) {
+    CU(cudaSetDevice(ctx->device));
+    if (s.shared_pending) { CU(cudaStreamWaitEvent(s.stream, s.ev_shared_done, 0)); s.shared_pending = false; }
+    if (!ctx->line_hint_fixed) ctx->line_hint = measure_line(static_cast<const char *>(host), nbytes, info ? (size_t)info->data_valid_from : 0);
+    if (nbytes) CU(cudaMemcpyAsync(s.d_in, host, nbytes, cudaMemcpyHostToDevice, s.stream));
+    CU(cudaMemsetAsync(s.d_in + nbytes, '\n', 64, s.stream));
+    CU(cudaEventRecord(s.ev_h2d, s.stream));
+    return start_chunk(ctx, s, s.d_in, nbytes, info);
+}
+
+// A launch that ran out of room says why in DevStats::overflow, and phase_checker / genotype_query may have dropped more
+// lines than the event list holds.  This grows what was short and returns 1 when the chunk is to run again (its input is
+// still on the device), 0 when the result stands (an overflow left in it is then an error), a negative vcfx_err on failure.
+// `out` is the slot whose output buffer may grow; the device-resident path passes null, since its caller owns that
+// buffer, and an OV_OUTPUT is final there.  The row records always get room for the count plus rec_slack: a re-run for
+// any reason may reserve that many more.
+static int grow_for_rerun(vcfx_ctx *ctx, Work &w, size_t max_bytes, Slot *out) {
+    const int grew = grow_events(ctx, w);
+    if (grew < 0) return grew;
+    const unsigned long long ov = w.h_stats->overflow & (out ? ~0ULL : ~(unsigned long long)OV_OUTPUT);
+    if (!ov && !grew) return 0;
+    if (ov & OV_AC_SPEC) ctx->ac_spec = false;
+    int rc = ensure_work(ctx, w, max_bytes, w.h_stats->n_recs + rec_slack(ctx), (ov & OV_IB_PANELS) ? ib_panel_need(ctx, w) : 0);
+    if (rc != VCFX_OK) return rc;
+    if (ov & OV_OUTPUT) {
+        const size_t want = std::max((size_t)w.h_stats->bytes_out + (1u << 20), out->out_cap + out->out_cap / 4);
+        cudaFree(out->d_out); cudaFreeHost(out->h_out); out->d_out = nullptr; out->h_out = nullptr; out->out_cap = 0;
+        CU(cudaMalloc(&out->d_out, want));
+        CU(cudaMallocHost(&out->h_out, want));
+        out->out_cap = want;
+    }
+    return 1;
+}
+
 int vcfx_cuda_acquire_input(vcfx_ctx *ctx, char **buf, size_t *cap) {
     if (!ctx || !buf || !cap) return VCFX_E_INVALID;
     if (ctx->acquired_slot >= 0) {           // re-acquire returns the same buffer
@@ -761,21 +798,9 @@ int vcfx_cuda_acquire_input(vcfx_ctx *ctx, char **buf, size_t *cap) {
 int vcfx_cuda_submit(vcfx_ctx *ctx, size_t nbytes, const vcfx_chunk_info *info) {
     if (!ctx || ctx->acquired_slot < 0 || nbytes > ctx->chunk_bytes) return VCFX_E_INVALID;
     Slot &s = ctx->slots[ctx->acquired_slot];
-    CU(cudaSetDevice(ctx->device));
-    if (s.shared_pending) { CU(cudaStreamWaitEvent(s.stream, s.ev_shared_done, 0)); s.shared_pending = false; }
-    if (!ctx->line_hint_fixed) ctx->line_hint = measure_line(s.h_in, nbytes, info ? (size_t)info->data_valid_from : 0);
-    if (nbytes) CU(cudaMemcpyAsync(s.d_in, s.h_in, nbytes, cudaMemcpyHostToDevice, s.stream));
-    CU(cudaMemsetAsync(s.d_in + nbytes, '\n', 64, s.stream));
-    CU(cudaEventRecord(s.ev_h2d, s.stream));
-    s.d_in_used = s.d_in;
-    if (info) s.info = *info; else s.info = vcfx_chunk_info{0, 1, 0, 0, 0};
-    ib_begin(ctx, s.w, &s.info);
-    int rc = launch_chunk(ctx, s.w, s.stream, s.d_in, nbytes, &s.info, s.d_out, s.out_cap, false);
+    int rc = upload_and_start(ctx, s, s.h_in, nbytes, info);
     if (rc != VCFX_OK) return rc;
-    s.nbytes = nbytes; s.in_flight = true; s.d2h_issued = false;
     ctx->acquired_slot = -1;
-    ctx->head = (ctx->head + 1) % ctx->n_slots;
-    ctx->n_in_flight++;
     kick_ready(ctx);
     return VCFX_OK;
 }
@@ -786,20 +811,8 @@ int vcfx_cuda_submit_host(vcfx_ctx *ctx, const void *host, size_t nbytes, const 
     Slot &s = ctx->slots[ctx->head];
     int rc = ensure_slot(ctx, s);
     if (rc != VCFX_OK) return rc;
-    CU(cudaSetDevice(ctx->device));
-    if (s.shared_pending) { CU(cudaStreamWaitEvent(s.stream, s.ev_shared_done, 0)); s.shared_pending = false; }
-    if (!ctx->line_hint_fixed) ctx->line_hint = measure_line(static_cast<const char *>(host), nbytes, info ? (size_t)info->data_valid_from : 0);
-    if (nbytes) CU(cudaMemcpyAsync(s.d_in, host, nbytes, cudaMemcpyHostToDevice, s.stream));
-    CU(cudaMemsetAsync(s.d_in + nbytes, '\n', 64, s.stream));
-    CU(cudaEventRecord(s.ev_h2d, s.stream));
-    s.d_in_used = s.d_in;
-    if (info) s.info = *info; else s.info = vcfx_chunk_info{0, 1, 0, 0, 0};
-    ib_begin(ctx, s.w, &s.info);
-    rc = launch_chunk(ctx, s.w, s.stream, s.d_in, nbytes, &s.info, s.d_out, s.out_cap, false);
+    rc = upload_and_start(ctx, s, host, nbytes, info);
     if (rc != VCFX_OK) return rc;
-    s.nbytes = nbytes; s.in_flight = true; s.d2h_issued = false;
-    ctx->head = (ctx->head + 1) % ctx->n_slots;
-    ctx->n_in_flight++;
     kick_ready(ctx);
     return VCFX_OK;
 }
@@ -821,29 +834,23 @@ int vcfx_cuda_submit_shared(vcfx_ctx *ctx, vcfx_ctx *primary, const vcfx_chunk_i
     if (rc != VCFX_OK) return rc;
     CU(cudaSetDevice(ctx->device));
     CU(cudaStreamWaitEvent(s.stream, ps.ev_h2d, 0));                 // the bytes are there
-    if (info) s.info = *info; else s.info = vcfx_chunk_info{0, 1, 0, 0, 0};
     // An operation that may have to run a chunk again (more rows or more text than its slot was sized for) takes a
     // private device copy (a few tens of microseconds): the primary is then free to reuse its buffer at once and a
     // re-run never reads bytes the primary has overwritten.  variant_counter never re-runs and reads the primary's bytes.
-    const bool own_copy = ctx->cfg.op != VCFX_OP_VARIANT_COUNT;
+    const bool own_copy = ctx->op->reruns;
     if (own_copy) {
         if (ps.nbytes) CU(cudaMemcpyAsync(s.d_in, ps.d_in, ps.nbytes, cudaMemcpyDeviceToDevice, s.stream));
         CU(cudaMemsetAsync(s.d_in + ps.nbytes, '\n', 64, s.stream));
         CU(cudaEventRecord(ps.ev_shared_done, s.stream));
         ps.shared_pending = true;
     }
-    s.d_in_used = own_copy ? s.d_in : ps.d_in;
-    ib_begin(ctx, s.w, &s.info);
-    rc = launch_chunk(ctx, s.w, s.stream, s.d_in_used, ps.nbytes, &s.info, s.d_out, s.out_cap, false);
+    rc = start_chunk(ctx, s, own_copy ? s.d_in : ps.d_in, ps.nbytes, info);
     if (rc != VCFX_OK) return rc;
     if (!own_copy) {
         // the primary may not overwrite that device buffer before this context has read it
         CU(cudaEventRecord(ps.ev_shared_done, s.stream));
         ps.shared_pending = true;
     }
-    s.nbytes = ps.nbytes; s.in_flight = true; s.d2h_issued = false;
-    ctx->head = (ctx->head + 1) % ctx->n_slots;
-    ctx->n_in_flight++;
     return VCFX_OK;
 }
 
@@ -857,29 +864,11 @@ int vcfx_cuda_next_output(vcfx_ctx *ctx, const char **text, size_t *n, vcfx_chun
     s.in_flight = false;
     ctx->tail = (ctx->tail + 1) % ctx->n_slots;
     ctx->n_in_flight--;
-    // A chunk with more rows / more text than the slot was sized for is simply run again with
-    // exact sizes (the input is still on the device); the larger buffers are kept, with headroom.
+    // a chunk with more rows / more text than the slot was sized for is run again; the larger buffers are kept
     for (int attempt = 0; attempt < 3; ++attempt) {
-        const int grew = grow_events(ctx, s.w);
-        if (grew < 0) return grew;
-        if (!s.w.h_stats->overflow && !grew) break;
-        const unsigned long long ov = s.w.h_stats->overflow;
-        if (ov & 4) ctx->ac_exact = true;
-        if (ov & 1) {
-            int rc = ensure_work(ctx, s.w, ctx->chunk_bytes, s.w.h_stats->n_recs + rec_slack(ctx));
-            if (rc != VCFX_OK) return rc;
-        }
-        if (ov & 16) {                  // inbreeding_calculator: more rows x samples than the panels hold (few columns per line)
-            int rc = ensure_work(ctx, s.w, ctx->chunk_bytes, 0, ib_panel_need(ctx, s.w));
-            if (rc != VCFX_OK) return rc;
-        }
-        if (ov & 2) {
-            const size_t want = std::max((size_t)s.w.h_stats->bytes_out + (1u << 20), s.out_cap + s.out_cap / 4);
-            cudaFree(s.d_out); cudaFreeHost(s.h_out); s.d_out = nullptr; s.h_out = nullptr; s.out_cap = 0;
-            CU(cudaMalloc(&s.d_out, want));
-            CU(cudaMallocHost(&s.h_out, want));
-            s.out_cap = want;
-        }
+        const int again = grow_for_rerun(ctx, s.w, ctx->chunk_bytes, &s);
+        if (again < 0) return again;
+        if (!again) break;
         int rc = launch_chunk(ctx, s.w, s.stream, s.d_in_used, s.nbytes, &s.info, s.d_out, s.out_cap, false);
         if (rc != VCFX_OK) return rc;
         CU(cudaStreamSynchronize(s.stream));
@@ -913,7 +902,7 @@ int vcfx_cuda_short_lines(vcfx_ctx *ctx, uint64_t *line_no, size_t cap, size_t *
 int vcfx_cuda_run_device(vcfx_ctx *ctx, void *d_in, size_t nbytes, const vcfx_chunk_info *info,
                          void *d_out, size_t out_cap) {
     if (!ctx || !d_in || ((uintptr_t)d_in & 15)) return VCFX_E_INVALID;
-    if (is_ds_matrix(ctx->cfg) && ((uintptr_t)d_out & 15)) return VCFX_E_INVALID;     // the row metadata is written in 16-byte stores
+    if (ctx->ds_matrix && ((uintptr_t)d_out & 15)) return VCFX_E_INVALID;     // the row metadata is written in 16-byte stores
     CU(cudaSetDevice(ctx->device));
     int rc = ensure_work(ctx, ctx->dev_work, nbytes);
     if (rc != VCFX_OK) return rc;
@@ -932,16 +921,12 @@ int vcfx_cuda_sync(vcfx_ctx *ctx, vcfx_chunk_stats *stats) {
     CU(cudaSetDevice(ctx->device));
     CU(cudaStreamSynchronize(ctx->dev_stream));
     ctx->dev_pending = false;
-    const int grew = grow_events(ctx, ctx->dev_work);
-    if (grew < 0) return grew;
-    if ((ctx->dev_work.h_stats->overflow & 29) || grew) {      // more rows than sized for / speculative row sizes off / more events: run again
-        if (ctx->dev_work.h_stats->overflow & 4) ctx->ac_exact = true;
-        int rc2 = ensure_work(ctx, ctx->dev_work, ctx->dev_nbytes, ctx->dev_work.h_stats->n_recs + rec_slack(ctx),
-                              (ctx->dev_work.h_stats->overflow & 16) ? ib_panel_need(ctx, ctx->dev_work) : 0);
-        if (rc2 != VCFX_OK) return rc2;
-        rc2 = launch_chunk(ctx, ctx->dev_work, ctx->dev_stream, ctx->dev_in, ctx->dev_nbytes, &ctx->dev_info,
-                           ctx->dev_out, ctx->dev_out_cap);
-        if (rc2 != VCFX_OK) return rc2;
+    const int again = grow_for_rerun(ctx, ctx->dev_work, ctx->dev_nbytes, nullptr);       // one re-run at most
+    if (again < 0) return again;
+    if (again) {
+        int rc = launch_chunk(ctx, ctx->dev_work, ctx->dev_stream, ctx->dev_in, ctx->dev_nbytes, &ctx->dev_info,
+                              ctx->dev_out, ctx->dev_out_cap);
+        if (rc != VCFX_OK) return rc;
         CU(cudaStreamSynchronize(ctx->dev_stream));
     }
     int rc = fetch_events(ctx, ctx->dev_work, ctx->dev_stream);

@@ -79,10 +79,20 @@ struct DevStats {
     unsigned long long dots_terminated;
     unsigned long long last_unterminated_flagged;
     unsigned long long bytes_out;
-    unsigned long long overflow;          // bit 0: row records, bit 1: output bytes, bit 2: speculative row sizes were wrong
+    unsigned long long overflow;          // OV_* bits: why the launch has to run again (vcfx_api.cu grows what they name)
     unsigned long long first_short_line;  // filled by tile_scan_kernel
     unsigned long long n_recs;            // row-record slots reserved (may exceed rec_cap: then overflow)
     unsigned long long n_unfinished;      // tiles the lattice kernel left to the general kernel
+};
+
+// DevStats::overflow.  A launch that sets any of them wrote nothing that can be used; the host grows what the bit names
+// and runs the chunk again (its input is still on the device)
+enum : unsigned long long {
+    OV_RECS = 1,          // more rows than row records (n_recs > rec_cap)
+    OV_OUTPUT = 2,        // more output bytes than out_cap (inbreeding_calculator: than text_cap)
+    OV_AC_SPEC = 4,       // allele_counter's speculative row sizes were wrong (a count of two digits): size rows by parsing
+    OV_IB_ORDER = 8,      // inbreeding_calculator: an earlier chunk is being run again, so this one has to be too
+    OV_IB_PANELS = 16,    // inbreeding_calculator: more rows x samples than the panels hold
 };
 
 // shared-memory event counters of K1: slot = index of the 64-bit field in DevStats
@@ -2117,7 +2127,7 @@ __device__ __forceinline__ bool tile_lines(const KParams &P, const WarpShared ws
                             // the write pass never stores past the bytes the size pass gave this tile (speculative sizes can be
                             // too small: a count of two digits) nor past the output buffer; the chunk is then run again, exact
                             if (P.ac_pass && opos + btot > out_limit) {
-                                if (lane == 0) atomicOr(&P.stats->overflow, 4ULL);
+                                if (lane == 0) atomicOr(&P.stats->overflow, (unsigned long long)OV_AC_SPEC);
                             } else
                             if (fast) {
                                 uint32_t *sw = reinterpret_cast<uint32_t *>(stage0);
@@ -2430,6 +2440,10 @@ __device__ __forceinline__ bool tile_lines(const KParams &P, const WarpShared ws
 #ifndef VCFX_GENERAL_CTAS
 #define VCFX_GENERAL_CTAS 3          // resident CTAs per SM of the general kernel: 80 registers, no spills (C3 allele_freq_calc 1.85 ms at 4 CTAs / 64 registers, 1.90 at 5 / 48, 1.72 at 3 / 80)
 #endif
+// resident CTAs per SM of vcfx_scan_kernel<OP, VAR>: its __launch_bounds__, and the grids vcfx_api.cu launches it with
+__host__ __device__ constexpr int scan_ctas(int op, int var) {
+    return (op == OP_VC) ? 5 : (var == 1 ? VCFX_GENERAL_CTAS : (op == OP_AC ? VCFX_AC_CTAS : VCFX_PARSE_CTAS));
+}
 // Two kernels for allele_freq_calc and hwe_tester, launched one after the other over the same tiles, so that each is
 // compiled (registers, schedule) on its own:
 //   VAR 0  the lattice kernel: tier 1 + the exact path.  In a tile it stops at the first line whose first sample
@@ -2439,7 +2453,7 @@ __device__ __forceinline__ bool tile_lines(const KParams &P, const WarpShared ws
 //          skip-ahead loop for multi-key FORMATs, tier 1 and the exact path); it exits at once when none was left
 // The other operations have one kernel (VAR 0, never stops early).
 template <int OP, int VAR>
-__global__ void __launch_bounds__(WARPS_PER_CTA * 32, (OP == OP_VC) ? 5 : (VAR == 1 ? VCFX_GENERAL_CTAS : (OP == OP_AC ? VCFX_AC_CTAS : VCFX_PARSE_CTAS)))
+__global__ void __launch_bounds__(WARPS_PER_CTA * 32, scan_ctas(OP, VAR))
 vcfx_scan_kernel(const VCFX_GRID_CONSTANT KParams P) {
     __shared__ uint32_t s_tp[WARPS_PER_CTA][12];
     __shared__ __align__(128) uint8_t s_ring[(VCFX_C4_RING && VAR == 1) ? WARPS_PER_CTA * C4_RING : 16];
@@ -2547,7 +2561,7 @@ vcfx_scan_kernel(const VCFX_GRID_CONSTANT KParams P) {
         }
         if (lane == 0 && !(OP == OP_AC && P.ac_pass)) { P.tile_lines[tile] = nlines; P.tile_out[tile] = out_bytes; }
         // the write pass of a speculatively sized launch checks the sizes it was given
-        if (OP == OP_AC && P.ac_pass && P.ac_spec && lane == 0 && (unsigned long long)out_bytes != P.tile_out[tile]) atomicOr(&P.stats->overflow, 4ULL);
+        if (OP == OP_AC && P.ac_pass && P.ac_spec && lane == 0 && (unsigned long long)out_bytes != P.tile_out[tile]) atomicOr(&P.stats->overflow, (unsigned long long)OV_AC_SPEC);
         __syncwarp();
         if (lane < CNT_SLOTS) {
             const unsigned int v = s_cnt[wid][lane];
@@ -2649,8 +2663,8 @@ tile_scan_kernel(const KParams P) {
         unsigned long long k = P.stats->first_short_key;
         P.stats->first_short_line = (k == ~0ULL) ? 0ULL : P.line_base[k >> 32] + (k & 0xFFFFFFFFULL) + 1ULL;
         unsigned long long ov = 0;
-        if (P.stats->n_recs > P.rec_cap) ov |= 1;
-        if (P.stats->bytes_out > P.out_cap) ov |= 2;
+        if (P.stats->n_recs > P.rec_cap) ov |= OV_RECS;
+        if (P.stats->bytes_out > P.out_cap) ov |= OV_OUTPUT;
         P.stats->overflow = ov;
     }
 }
@@ -2885,7 +2899,7 @@ ib_rows_kernel(const KParams P) {
     const unsigned long long R = P.stats->bytes_out;                 // rows of the chunk (tile_scan_kernel's total)
     const uint32_t npan = (P.n_sel + 31u) >> 5;
     if (R * 32ULL * npan > P.ib_panel_cap) {                         // (every thread sees the same: nobody writes)
-        if (blockIdx.x == 0 && threadIdx.x == 0) atomicOr(&P.stats->overflow, 16ULL);
+        if (blockIdx.x == 0 && threadIdx.x == 0) atomicOr(&P.stats->overflow, (unsigned long long)OV_IB_PANELS);
         return;
     }
     const int lane = threadIdx.x & 31;
@@ -3209,7 +3223,7 @@ ib_finish_kernel(const KParams P) {
         int st = 0;                                                  // 0 = go on, 1 = leave
         if (P.stats->overflow) st = 1;
         else if (S.seq == P.ib_seq) S.seq = P.ib_seq + 1;            // this launch applied the chunk
-        else if (S.seq != P.ib_seq + 1) { P.stats->overflow = 8; st = 1; }   // an earlier chunk is being run again: so will this one
+        else if (S.seq != P.ib_seq + 1) { P.stats->overflow = OV_IB_ORDER; st = 1; }   // an earlier chunk is being run again: so will this one
         if (st || !P.is_final) P.stats->bytes_out = 0;
         s_state = st; s_carry = 0;
     }
@@ -3255,7 +3269,7 @@ ib_finish_kernel(const KParams P) {
     }
     if (tid == 0) {
         P.stats->bytes_out = s_carry;
-        if (s_carry > P.text_cap) P.stats->overflow = 2;
+        if (s_carry > P.text_cap) P.stats->overflow = OV_OUTPUT;
     }
 }
 
