@@ -6,7 +6,8 @@ the fraction of the measured HBM peak.
 
   C2  427,409 x 2,504 phased GT                      allele_freq_calc, variant_counter, hwe_tester
   C3  C2 shape + 5 % missing / unphased / haploid    missing_detector, allele_counter (TEXT, -a), allele_freq_calc
-  C2, C3 also: dosage_calculator as text and as its int8 matrix (dosage_matrix, VCFX_F_DS_MATRIX, width = S)
+  C2, C3 also: dosage_calculator as text, as its int8 matrix (dosage_matrix, VCFX_F_DS_MATRIX, width = S) and as
+              PLINK 1 .bed rows (dosage_bed, VCFX_F_DS_BED, width = S)
   C4  GT:AD:DP:GQ:PL multi-allelic (scaled to ~4 GB) hwe_tester, allele_freq_calc
 """
 from __future__ import annotations
@@ -46,11 +47,11 @@ def main():
         "C2": (2, int(427409 * args.scale), [("allele_freq_calc", api.OP_ALLELE_FREQ, 0), ("variant_counter", api.OP_VARIANT_COUNT, 0),
                                              ("hwe_tester", api.OP_HWE, 0), ("nonref_filter", api.OP_NONREF_FILTER, 0), ("phase_checker", api.OP_PHASE_CHECK, 0),
                                              ("indexer", api.OP_INDEX, 0), ("inbreeding_calculator", api.OP_INBREEDING, 0), ("genotype_query", api.OP_GENOTYPE_QUERY, 0), ("dosage_calculator", api.OP_DOSAGE, 0),
-                                             ("dosage_matrix", api.OP_DOSAGE, api.F_DS_MATRIX)]),
+                                             ("dosage_matrix", api.OP_DOSAGE, api.F_DS_MATRIX), ("dosage_bed", api.OP_DOSAGE, api.F_DS_BED)]),
         "C3": (3, int(427409 * args.scale), [("missing_detector", api.OP_MISSING_DETECT, 0), ("allele_counter -a", api.OP_ALLELE_COUNT, api.F_AC_AGGREGATE),
                                              ("allele_counter", api.OP_ALLELE_COUNT, 0), ("allele_freq_calc", api.OP_ALLELE_FREQ, 0),
                                              ("inbreeding_calculator", api.OP_INBREEDING, 0), ("dosage_calculator", api.OP_DOSAGE, 0),
-                                             ("dosage_matrix", api.OP_DOSAGE, api.F_DS_MATRIX)]),
+                                             ("dosage_matrix", api.OP_DOSAGE, api.F_DS_MATRIX), ("dosage_bed", api.OP_DOSAGE, api.F_DS_BED)]),
         "C4": (4, int(60000 * args.scale), [("hwe_tester", api.OP_HWE, 0), ("allele_freq_calc", api.OP_ALLELE_FREQ, 0)]),
     }
     for cname in args.configs.split(","):
@@ -79,6 +80,8 @@ def main():
                 out_cap = int(nbytes * 9.5) + (1 << 20)
             if op == api.OP_DOSAGE and flags == api.F_DS_MATRIX:
                 out_cap = (V + hdr.count(b"\n") + 1) * (16 + S)          # rows <= lines, 16 + W bytes a row
+            if op == api.OP_DOSAGE and flags == api.F_DS_BED:
+                out_cap = (V + hdr.count(b"\n") + 1) * (16 + (S + 3) // 4)
             d_out = torch.empty(out_cap, dtype=torch.uint8, device=dev)
             kw = dict(sel_cols=list(range(S)), sel_names=names) if op in (api.OP_ALLELE_COUNT, api.OP_INBREEDING) else (dict(query=b"1/1") if op == api.OP_GENOTYPE_QUERY
                                                                                                                    else dict(width=S) if (op == api.OP_DOSAGE and flags) else {})

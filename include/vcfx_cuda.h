@@ -72,7 +72,16 @@ typedef enum {
                                      column of a line without a GT key too), -2 for a column s >= n_cols the line does not have.
                                      Columns beyond W are dropped (n_cols keeps the true count; stats.flagged counts such rows).
                                      stats.rows = rows, stats.bytes_out = rows x (16 + W); short_lines, data_lines as for the text.
-                                     run_device wants d_out 16-byte aligned (else VCFX_E_INVALID) */
+                                     run_device wants d_out 16-byte aligned (else VCFX_E_INVALID).
+                                     VCFX_F_DS_BED: the same rows as PLINK 1 .bed rows (variant-major), W = cfg.n_sel (0 is
+                                     valid), B = ceil(W / 4) bytes a row.  Output: rows x vcfx_ds_row, then at byte 16 x rows
+                                     the rows x B packed bytes, row-major; stats.bytes_out = rows x (16 + B), stats.flagged
+                                     as for the matrix.  Sample s sits in byte s >> 2 at bits 2 (s & 3) and 2 (s & 3) + 1, with
+                                     A1 = ALT and A2 = REF: matrix code 2 -> 00 (hom A1), 1 -> 10 (het), 0 -> 11 (hom A2),
+                                     -1 and -2 -> 01 (missing), s >= W -> 00 (padding).  A multi-allelic line keeps the
+                                     dosage rule (every allele > 0 counts): A1 stands for "any non-REF allele".  Cannot be
+                                     combined with VCFX_F_DS_MATRIX (VCFX_E_INVALID from create); run_device wants d_out
+                                     16-byte aligned */
     VCFX_OP_INDEX          = 6,   /* VCFX_indexer.cpp:205-322 createVCFIndexMmap, :329-443 createVCFIndex (SURVEY §8 f4) */
     VCFX_OP_NONREF_FILTER  = 5    /* VCFX_nonref_filter.cpp:458-548 filterNonRefMmap, :553-631 filterNonRef (SURVEY §8 f2) */
 } vcfx_op;
@@ -102,6 +111,7 @@ typedef enum {
 #define VCFX_F_AC_AGGREGATE   0x01u  /* -a: one row per variant (countAllelesUnified :1440-1461)          */
 #define VCFX_F_AC_BINARY      0x02u  /* -b: int8 {ref,alt} per selected sample (:1444-1449)               */
 #define VCFX_F_DS_MATRIX      0x01u  /* dosage_calculator: int8 variants x samples matrix instead of text (see VCFX_OP_DOSAGE) */
+#define VCFX_F_DS_BED         0x02u  /* dosage_calculator: PLINK 1 .bed rows, 2 bits a call, instead of text (see VCFX_OP_DOSAGE) */
 #define VCFX_F_AC_FORWARD     0x04u  /* stdin / unified column walk: forward only, stop at the first absent
                                         column (:1222-1229, :1416-1423); without it: processChunk's random
                                         access with 0/0 padding and int8 storage (:610-627)               */
@@ -124,7 +134,7 @@ typedef struct {
     const uint32_t *sel_name_off;   /* [n_sel + 1] offsets into sel_names                       */
 } vcfx_cfg;
 
-/* VCFX_OP_DOSAGE with VCFX_F_DS_MATRIX: the metadata of one matrix row (16 bytes, the rows in file order) */
+/* VCFX_OP_DOSAGE with VCFX_F_DS_MATRIX or VCFX_F_DS_BED: the metadata of one row (16 bytes, the rows in file order) */
 typedef struct vcfx_ds_row {
     uint64_t line_offset;      /* offset of the row's line in the whole input: info.file_offset + offset in the chunk */
     uint32_t n_cols;           /* sample columns of the line (may exceed W)                                           */

@@ -600,8 +600,9 @@ def dosage_calculator(data: bytes, mode: int = FILE, quiet: bool = False, chunk_
     return ToolResult(DS_HEADER + body, 0, tot, warn)
 
 
-F_DS_MATRIX = 1
+F_DS_MATRIX, F_DS_BED = 1, 2
 DS_ROW_BYTES = 16                                      # vcfx_ds_row: uint64 line_offset, uint32 n_cols, uint32 flags
+BED_MAGIC = b"\x6c\x1b\x01"                            # PLINK 1 .bed: the two magic bytes, then 01 = variant-major
 
 
 @dataclass
@@ -618,6 +619,22 @@ class DosageMatrix:
     err: bytes = b""               # the warnings the tool prints on stderr
 
 
+@dataclass
+class DosageBed:
+    """The same rows as PLINK 1 .bed rows (variant-major, A1 = ALT, A2 = REF): packed[i] holds the calls of row i, sample s
+    at bits 2 (s & 3) of byte s >> 2 — 00 dosage 2 (on a multi-allelic line: two non-REF alleles), 10 dosage 1, 11
+    dosage 0, 01 missing ("NA", no GT key, or no column s), 00 padding from the width on.  BED_MAGIC followed by the rows
+    of packed is a .bed file."""
+    samples: list                  # the "#CHROM" line's columns from index 9
+    width: int                     # W: samples per row
+    packed: object                 # uint8 [rows, ceil(W / 4)]
+    line_offset: object            # int64 [rows]
+    n_cols: object                 # int32 [rows]
+    no_gt: object                  # bool [rows]
+    totals: Totals
+    err: bytes = b""
+
+
 def _ds_matrix_prescan(data, mode: int):
     """(sample names) after dosage_calculator's host rule: a data line in front of the "#CHROM" line ends the tool's run."""
     first_data, found, names = _ds_prescan(data, mode)
@@ -626,34 +643,61 @@ def _ds_matrix_prescan(data, mode: int):
     return names
 
 
-def _ds_split(piece: bytes, width: int):
-    """(metadata, codes) numpy views of one chunk's matrix output."""
+def _ds_row_bytes(flags: int, width: int) -> int:
+    """Bytes of a row behind its metadata: W int8 codes, or ceil(W / 4) packed .bed bytes."""
+    return (width + 3) // 4 if flags & F_DS_BED else width
+
+
+def _ds_split(piece: bytes, width: int, flags: int = F_DS_MATRIX):
+    """(metadata, codes or packed bytes) numpy views of one chunk's matrix or .bed output."""
     import numpy as np
-    rows = len(piece) // (DS_ROW_BYTES + width)
+    nb = _ds_row_bytes(flags, width)
+    rows = len(piece) // (DS_ROW_BYTES + nb)
     meta = np.frombuffer(piece, dtype=np.dtype([("line_offset", "<u8"), ("n_cols", "<u4"), ("flags", "<u4")]), count=rows)
-    codes = np.frombuffer(piece, dtype=np.int8, count=rows * width, offset=DS_ROW_BYTES * rows).reshape(rows, width)
-    return meta, codes
+    body = np.frombuffer(piece, dtype=np.uint8 if flags & F_DS_BED else np.int8, count=rows * nb, offset=DS_ROW_BYTES * rows)
+    return meta, body.reshape(rows, nb)
+
+
+def _ds_host(data, mode: int, width, chunk_bytes: int, flags: int, kw):
+    """One stream of host bytes in the matrix or .bed layout: (names, W, metadata, rows of codes or packed bytes, Totals)."""
+    import numpy as np
+    names = [] if (mode == FILE and len(data) == 0) else _ds_matrix_prescan(data, mode)
+    W = len(names) if width is None else int(width)
+    metas, bodies, tot = [], [], Totals()
+    if len(data):
+        outs, tot = _stream(OP_DOSAGE, data, mode, chunk_bytes, flags=flags, width=W, **kw)
+        for piece in outs:
+            m, b = _ds_split(piece, W, flags)
+            metas.append(m); bodies.append(b)
+    empty = _ds_split(b"", W, flags)
+    meta = np.concatenate(metas) if metas else empty[0]
+    body = np.ascontiguousarray(np.concatenate(bodies)) if bodies else empty[1].copy()
+    return names, W, meta, body, tot
+
+
+def _ds_meta_host(meta):
+    """line_offset, n_cols, no_gt as CPU tensors."""
+    import numpy as np
+    import torch
+    return (torch.from_numpy(meta["line_offset"].astype(np.int64)), torch.from_numpy(meta["n_cols"].astype(np.int32)),
+            torch.from_numpy((meta["flags"] & 1).astype(bool)))
 
 
 def dosage_matrix(data: bytes, mode: int = FILE, width: int | None = None, chunk_bytes: int = 0, **kw) -> DosageMatrix:
     """dosage_calculator's genotypes as an int8 variants x samples matrix (CPU tensors), through the streaming path.  The
     width defaults to the number of samples of the "#CHROM" line.  Raises VcfxCudaError with the tool's error text when a
     data line comes before the "#CHROM" line."""
-    import numpy as np
     import torch
-    names = [] if (mode == FILE and len(data) == 0) else _ds_matrix_prescan(data, mode)
-    W = len(names) if width is None else int(width)
-    metas, codes, tot = [], [], Totals()
-    if len(data):
-        outs, tot = _stream(OP_DOSAGE, data, mode, chunk_bytes, flags=F_DS_MATRIX, width=W, **kw)
-        for piece in outs:
-            m, c = _ds_split(piece, W)
-            metas.append(m); codes.append(c)
-    meta = np.concatenate(metas) if metas else _ds_split(b"", W)[0]
-    code = np.concatenate(codes) if codes else np.zeros((0, W), dtype=np.int8)
-    return DosageMatrix(names, torch.from_numpy(np.ascontiguousarray(code)), torch.from_numpy(meta["line_offset"].astype(np.int64)),
-                        torch.from_numpy(meta["n_cols"].astype(np.int32)), torch.from_numpy((meta["flags"] & 1).astype(bool)),
-                        tot, DS_WARNING * tot.short_lines)
+    names, W, meta, code, tot = _ds_host(data, mode, width, chunk_bytes, F_DS_MATRIX, kw)
+    return DosageMatrix(names, torch.from_numpy(code), *_ds_meta_host(meta), tot, DS_WARNING * tot.short_lines)
+
+
+def dosage_bed(data: bytes, mode: int = FILE, width: int | None = None, chunk_bytes: int = 0, **kw) -> DosageBed:
+    """dosage_calculator's genotypes as PLINK 1 .bed rows (CPU tensors), through the streaming path; otherwise as
+    dosage_matrix.  BED_MAGIC + packed.numpy().tobytes() is the .bed file of the rows."""
+    import torch
+    names, W, meta, packed, tot = _ds_host(data, mode, width, chunk_bytes, F_DS_BED, kw)
+    return DosageBed(names, W, torch.from_numpy(packed), *_ds_meta_host(meta), tot, DS_WARNING * tot.short_lines)
 
 
 def _ds_device_head(d_in, nbytes: int, mode: int):
@@ -668,26 +712,24 @@ def _ds_device_head(d_in, nbytes: int, mode: int):
         k = min(nbytes, 4 * k)
 
 
-def dosage_matrix_device(d_in, nbytes: int, mode: int = FILE, width: int | None = None, line_hint: int = 0) -> DosageMatrix:
-    """dosage_matrix for an input already on the device: d_in is a uint8 CUDA tensor of at least nbytes + DEVICE_PAD bytes
-    (16-byte aligned).  Only the leading '#' block comes back to the host.  The output is sized from a newline count on
-    the device (rows <= lines) and the library runs on torch.cuda.current_stream(), so torch work behind it is ordered
-    after it; codes, line_offset, n_cols and no_gt are views into one output tensor on the same device."""
+def _ds_device(d_in, nbytes: int, mode: int, width, line_hint: int, flags: int):
+    """One resident launch in the matrix or .bed layout on torch's current stream: (names, W, metadata views, rows of codes
+    or packed bytes as a uint8 view, Totals), the views into one output tensor."""
     import torch
     if d_in.dtype != torch.uint8 or not d_in.is_cuda or d_in.numel() < nbytes + DEVICE_PAD or d_in.data_ptr() % 16:
         raise VcfxCudaError(-1, "d_in must be a 16-byte aligned uint8 CUDA tensor of at least nbytes + DEVICE_PAD bytes")
     names = [] if (mode == FILE and nbytes == 0) else _ds_device_head(d_in, nbytes, mode)
     W = len(names) if width is None else int(width)
+    nb = _ds_row_bytes(flags, W)
     lines = 1
     for s in range(0, nbytes, 1 << 28):                     # (bounded temporaries for inputs of several GB)
         lines += int((d_in[s:min(nbytes, s + (1 << 28))] == 10).sum())
-    row = DS_ROW_BYTES + W
-    out = torch.empty(max(lines * row, DS_ROW_BYTES), dtype=torch.uint8, device=d_in.device)
+    out = torch.empty(max(lines * (DS_ROW_BYTES + nb), DS_ROW_BYTES), dtype=torch.uint8, device=d_in.device)
     stream = torch.cuda.current_stream(d_in.device)
     tot = Totals()
     rows = 0
     if nbytes:
-        with Context(OP_DOSAGE, mode, device=d_in.device.index or 0, flags=F_DS_MATRIX, width=W, stream=stream.cuda_stream) as ctx:
+        with Context(OP_DOSAGE, mode, device=d_in.device.index or 0, flags=flags, width=W, stream=stream.cuda_stream) as ctx:
             if line_hint:
                 ctx.set_line_hint(line_hint)
             ctx.run_device(d_in.data_ptr(), nbytes, out.data_ptr(), out.numel())
@@ -695,9 +737,25 @@ def dosage_matrix_device(d_in, nbytes: int, mode: int = FILE, width: int | None 
         tot.add(st, 0, [])
         rows = int(st.rows)
     meta = out[:DS_ROW_BYTES * rows].view(rows, DS_ROW_BYTES)
-    return DosageMatrix(names, out[DS_ROW_BYTES * rows:DS_ROW_BYTES * rows + rows * W].view(torch.int8).view(rows, W),
-                        meta.view(torch.int64)[:, 0], meta.view(torch.int32)[:, 2], meta[:, 12].view(torch.bool),
-                        tot, DS_WARNING * tot.short_lines)
+    body = out[DS_ROW_BYTES * rows:DS_ROW_BYTES * rows + rows * nb].view(rows, nb)
+    return names, W, (meta.view(torch.int64)[:, 0], meta.view(torch.int32)[:, 2], meta[:, 12].view(torch.bool)), body, tot
+
+
+def dosage_matrix_device(d_in, nbytes: int, mode: int = FILE, width: int | None = None, line_hint: int = 0) -> DosageMatrix:
+    """dosage_matrix for an input already on the device: d_in is a uint8 CUDA tensor of at least nbytes + DEVICE_PAD bytes
+    (16-byte aligned).  Only the leading '#' block comes back to the host.  The output is sized from a newline count on
+    the device (rows <= lines) and the library runs on torch.cuda.current_stream(), so torch work behind it is ordered
+    after it; codes, line_offset, n_cols and no_gt are views into one output tensor on the same device."""
+    import torch
+    names, W, meta, body, tot = _ds_device(d_in, nbytes, mode, width, line_hint, F_DS_MATRIX)
+    return DosageMatrix(names, body.view(torch.int8), *meta, tot, DS_WARNING * tot.short_lines)
+
+
+def dosage_bed_device(d_in, nbytes: int, mode: int = FILE, width: int | None = None, line_hint: int = 0) -> DosageBed:
+    """dosage_bed for an input already on the device, as dosage_matrix_device: packed, line_offset, n_cols and no_gt are
+    views into one output tensor on the same device, written on torch.cuda.current_stream()."""
+    names, W, meta, body, tot = _ds_device(d_in, nbytes, mode, width, line_hint, F_DS_BED)
+    return DosageBed(names, W, body, *meta, tot, DS_WARNING * tot.short_lines)
 
 
 F_GQ_STRICT = 1

@@ -17,6 +17,7 @@
 using namespace vcfx;
 
 static_assert(sizeof(vcfx_ds_row) == 16, "ds_matrix_kernel writes a row's metadata as one 16-byte store");
+static_assert((VCFX_F_DS_MATRIX & VCFX_F_DS_BED) == 0, "the two dosage row layouts are separate bits");
 
 // kernel launches go through one macro so that the test-only warp emulator (tests/emu/) can build this file with g++
 #ifndef VCFX_LAUNCH
@@ -75,7 +76,8 @@ constexpr OpInfo OPS[] = {
     {vcfx_scan_kernel<OP_GQ, 0>,  nullptr,                    md_copy_kernel,              true,  true,  false, false, true,
      [](unsigned, size_t c) -> size_t { return c + 4096; }},
     // text: a sample column of two bytes or more gives at most two.  Matrix: a row takes 16 + W bytes, no more than its line
-    // when the line has W columns of two bytes or more (W >= 7); rows of fewer columns grow the slot once
+    // when the line has W columns of two bytes or more (W >= 7); .bed: 16 + ceil(W / 4), less still; rows of fewer columns
+    // grow the slot once
     {vcfx_scan_kernel<OP_DS, 0>,  nullptr,                    ds_rows_kernel,              false, false, false, true,  true,
      [](unsigned, size_t c) -> size_t { return c + 4096; }},
 };
@@ -134,7 +136,8 @@ struct vcfx_ctx {
     const OpInfo *op = nullptr;          // OPS[cfg.op]
     kernel_fn format = nullptr;          // the row writer launched behind the scan (op->format, or allele_counter's / the matrix's)
     bool two_pass = false;               // allele_counter text / binary: rows are sized in a first scan and written in a second
-    bool ds_matrix = false;              // dosage_calculator with VCFX_F_DS_MATRIX
+    bool ds_matrix = false;              // dosage_calculator with VCFX_F_DS_MATRIX or VCFX_F_DS_BED: rows of 16 + ds_row_bytes
+    uint64_t ds_row_bytes = 0;           // W (int8 matrix) or ceil(W / 4) (.bed)
     int device = 0;
     int sm_count = 0;
     int blocks_per_sm = 1;
@@ -394,7 +397,7 @@ int launch_chunk(vcfx_ctx *ctx, Work &w, cudaStream_t st, uint8_t *d_in, size_t 
     P.ib_codes = w.ib_codes; P.ib_rows = w.ib_rows; P.ib_panels = w.ib_panels; P.ib_panel_cap = w.ib_panel_cap; P.ib = ctx->d_ib; P.ib_seq = w.ib_seq; P.ib_first = w.ib_first ? 1 : 0; P.text_cap = out_cap;
     if (ctx->d_ib) P.out_cap = ~0ULL;       // the scan counts rows there, not bytes of text
     P.ds_matrix = ctx->ds_matrix ? 1 : 0;
-    P.unit_bytes = P.ds_matrix ? 16u + (uint64_t)ctx->n_sel : 1u;   // matrix mode: rows x (16 + W) <= out_cap once the rows are counted
+    P.unit_bytes = P.ds_matrix ? 16u + ctx->ds_row_bytes : 1u;      // matrix / .bed: rows x (16 + R) <= out_cap once the rows are counted
     P.stats = w.d_stats; P.events = w.events; P.ev_cap = w.ev_cap; P.ev_raw = op.raw_events ? 1 : 0;
 
     CU(cudaEventRecord(w.ev_k0, st));
@@ -630,10 +633,13 @@ int vcfx_cuda_create(const vcfx_cfg *cfg, vcfx_ctx **out) {
         CUC(cudaEventCreateWithFlags(&ctx->ib_event, cudaEventDisableTiming));
         if (!cfg->out_bytes) ctx->out_bytes = nb + (size_t)cfg->n_sel * 48 + 4096;      // "name \t F \n" per sample
     }
-    if (cfg->op == VCFX_OP_DOSAGE && (cfg->flags & VCFX_F_DS_MATRIX)) {
+    if (cfg->op == VCFX_OP_DOSAGE && (cfg->flags & (VCFX_F_DS_MATRIX | VCFX_F_DS_BED))) {
+        const bool bed = (cfg->flags & VCFX_F_DS_BED) != 0;
+        if (bed && (cfg->flags & VCFX_F_DS_MATRIX)) return fail(VCFX_E_INVALID);
         ctx->ds_matrix = true;
-        ctx->format = ds_matrix_kernel;
+        ctx->format = bed ? ds_matrix_kernel<true> : ds_matrix_kernel<false>;
         ctx->n_sel = cfg->n_sel;                                    // W, the sample columns of the matrix (0 is valid)
+        ctx->ds_row_bytes = bed ? ((uint64_t)cfg->n_sel + 3) / 4 : cfg->n_sel;
     }
     if (cfg->stream) { ctx->dev_stream = (cudaStream_t)cfg->stream; ctx->dev_stream_owned = false; }
     else { CUC(cudaStreamCreateWithFlags(&ctx->dev_stream, cudaStreamNonBlocking)); ctx->dev_stream_owned = true; }

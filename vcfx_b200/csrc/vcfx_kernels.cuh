@@ -160,9 +160,10 @@ struct KParams {
     int32_t ib_first;                // first chunk of a stream: the per-sample state starts from zero
     uint64_t text_cap;               // bytes the final text may take in out (out_cap is not compared with the row count)
     int32_t ev_raw;                  // 1: events are final values (phase_checker: line offset << 2 | kind), not (tile, index) keys
-    // DOSAGE matrix mode (VCFX_F_DS_MATRIX): a row is one unit of tile output (tile_base + off_in_tile = its rank), n_sel = W
+    // DOSAGE matrix and .bed modes (VCFX_F_DS_MATRIX, VCFX_F_DS_BED): a row is one unit of tile output (tile_base +
+    // off_in_tile = its rank), n_sel = W
     int32_t ds_matrix;
-    uint64_t unit_bytes;             // output bytes per unit of tile output: 1, or 16 + W in matrix mode (tile_scan_kernel's bytes_out)
+    uint64_t unit_bytes;             // output bytes per unit of tile output: 1, or 16 + W (matrix) / 16 + ceil(W / 4) (.bed) (tile_scan_kernel's bytes_out)
 };
 
 // ---------------------------------------------------------------------------------------
@@ -3021,11 +3022,14 @@ ds_rows_kernel(const KParams P) {
     }
 }
 
-// dosage_calculator matrix mode (VCFX_F_DS_MATRIX), K2b: a warp per row record.  The output is rows x 16 B of metadata
-// {uint64 line offset, uint32 columns, uint32 flags} followed by the rows x W int8 codes, row `rank` at 16 rows + rank W:
-// 0 / 1 / 2 the dosage, -1 "NA" (IB_NONE, IB_ABSENT, every column of a line without a GT key), -2 no such column.
-// A row is put together in shared memory at the destination's offset modulo 16, DSM_STEP samples at a time, and leaves in
-// aligned 128-bit stores; every lane builds 16 staged bytes from five aligned 32-bit loads of the codes.
+// dosage_calculator matrix mode (VCFX_F_DS_MATRIX) and .bed mode (VCFX_F_DS_BED), K2b: a warp per row record.  The output
+// is rows x 16 B of metadata {uint64 line offset, uint32 columns, uint32 flags} followed by rows of R bytes, row `rank` at
+// 16 rows + rank R.  Matrix (R = W): int8 codes, 0 / 1 / 2 the dosage, -1 "NA" (IB_NONE, IB_ABSENT, every column of a line
+// without a GT key), -2 no such column.  .bed (R = ceil(W / 4)): PLINK 1's two bits per sample, sample s at bits 2 (s & 3)
+// of byte s >> 2: 00 dosage 2, 10 dosage 1, 11 dosage 0, 01 missing (the matrix's -1 and -2), 00 padding from W on.
+// A row is put together in shared memory at the destination's offset modulo 16, DSM_STEP bytes at a time, and leaves in
+// aligned 128-bit stores.  Every lane reads 16 samples' codes with five aligned 32-bit loads, funnel-shifted to the row's
+// phase, so that a warp's loads cover consecutive words: they give 16 staged bytes of the matrix, or 4 of the .bed.
 constexpr uint32_t DSM_STAGE = 2048, DSM_STEP = DSM_STAGE - 16;     // DSM_STEP is a multiple of 16: every step has the same phase
 __device__ __forceinline__ uint32_t ds_matrix_word(uint32_t q, int s0, uint32_t ncols, bool no_gt) {
     const uint32_t na = ((q >> 2) | (q & (q >> 1))) & 0x01010101u;    // bytes holding IB_NONE (3) or IB_ABSENT (4)
@@ -3039,6 +3043,58 @@ __device__ __forceinline__ uint32_t ds_matrix_word(uint32_t q, int s0, uint32_t 
     }
     return w;
 }
+// 16 int8 codes, samples s0 .. s0 + 15
+__device__ __forceinline__ uint4 ds_matrix_lane(const uint8_t *codes, int s0, int sh, uint32_t ncols, bool no_gt) {
+    const int t0 = s0 - sh;                                                // sample of the aligned word that holds s0
+    uint32_t w[5];
+#pragma unroll
+    for (int j = 0; j < 5; ++j) {
+        const int t = t0 + 4 * j;
+        w[j] = (!no_gt && t + 3 >= 0 && t < (int)ncols) ? ldw(codes + t) : 0u;
+    }
+    uint4 o;
+    o.x = ds_matrix_word(__funnelshift_r(w[0], w[1], 8u * sh), s0, ncols, no_gt);
+    o.y = ds_matrix_word(__funnelshift_r(w[1], w[2], 8u * sh), s0 + 4, ncols, no_gt);
+    o.z = ds_matrix_word(__funnelshift_r(w[2], w[3], 8u * sh), s0 + 8, ncols, no_gt);
+    o.w = ds_matrix_word(__funnelshift_r(w[3], w[4], 8u * sh), s0 + 12, ncols, no_gt);
+    return o;
+}
+__device__ __forceinline__ uint32_t byte_mask(int n) {                // the low min(max(n, 0), 4) bytes
+    return n >= 4 ? 0xFFFFFFFFu : (n <= 0 ? 0u : (1u << (8 * n)) - 1u);
+}
+// four codes (one byte each, samples s .. s + 3) -> one .bed byte.  Code 0 -> 11, 1 -> 10, 2 -> 00, 3 / 4 -> 01: per byte
+// the low bit is b2 | !(b0 ^ b1) and the high bit !(b1 | b2) (codes are 0 .. 4).  Samples from ncols on are 01, from W on
+// 00 (EDGE = false: all four are below ncols).  One multiply gathers the four 2-bit fields: the field of byte j lands at
+// bits 24 + 2j, and the other partial products stay below bit 24 without overlapping.
+template <bool EDGE>
+__device__ __forceinline__ uint32_t ds_bed_byte(uint32_t q, int s, uint32_t ncols, uint32_t W) {
+    uint32_t m = (((q >> 2) | ~(q ^ (q >> 1))) & 0x01010101u) | ((~((q >> 1) | (q >> 2)) & 0x01010101u) << 1);
+    if (EDGE) {
+        const uint32_t keep_c = byte_mask((int)ncols - s), keep_w = byte_mask((int)W - s);
+        m = ((m & keep_c) | (0x01010101u & ~keep_c)) & keep_w;
+    }
+    return (m * 0x01041040u) >> 24;
+}
+// 4 .bed bytes, samples s0 .. s0 + 15 (s0 a multiple of 4)
+template <bool EDGE>
+__device__ __forceinline__ uint32_t ds_bed_lane(const uint8_t *codes, int s0, int sh, uint32_t ncols, uint32_t W) {
+    const int t0 = s0 - sh;
+    uint32_t w[5];
+#pragma unroll
+    for (int j = 0; j < 5; ++j) {
+        const int t = t0 + 4 * j;
+        w[j] = (!EDGE || (t + 3 >= 0 && t < (int)ncols)) ? ldw(codes + t) : 0u;
+    }
+    uint32_t o = 0;
+#pragma unroll
+    for (int j = 0; j < 4; ++j)
+        o |= ds_bed_byte<EDGE>(__funnelshift_r(w[j], w[j + 1], 8u * sh), s0 + 4 * j, ncols, W) << (8 * j);
+    return o;
+}
+// One kernel for both layouts: the record walk, the metadata, the staging and the flush are the same, only the per-lane
+// builder, its number of staged bytes and the row length differ (a compile-time choice: the matrix kernel's code is
+// what it was).
+template <bool BED>
 __global__ void __launch_bounds__(256)
 ds_matrix_kernel(const KParams P) {
     __shared__ __align__(16) uint8_t s_stage[8][DSM_STAGE];
@@ -3046,6 +3102,8 @@ ds_matrix_kernel(const KParams P) {
     const int lane = threadIdx.x & 31;
     uint8_t *stage = s_stage[threadIdx.x >> 5];
     const uint32_t W = P.n_sel;
+    const uint32_t R = BED ? (W >> 2) + ((W & 3u) != 0u) : W;              // bytes of a row
+    constexpr uint32_t LB = BED ? 4u : 16u;                                 // staged bytes a lane builds at a time
     const unsigned long long rows = P.stats->rows;
     uint8_t *const mat = P.out + 16ULL * rows;
     const unsigned long long nrec = P.stats->n_recs;
@@ -3059,30 +3117,25 @@ ds_matrix_kernel(const KParams P) {
             const unsigned long long off = P.file_offset + line;
             *reinterpret_cast<uint4 *>(P.out + 16ULL * rank) = make_uint4((uint32_t)off, (uint32_t)(off >> 32), r.a, r.c);
         }
-        if (W == 0) continue;
-        uint8_t *const dst = mat + rank * (unsigned long long)W;              // past 2^32 for realistic shapes
+        if (R == 0) continue;
+        uint8_t *const dst = mat + rank * (unsigned long long)R;              // past 2^32 for realistic shapes
         const uint8_t *const codes = P.ib_codes + ((line & ~3ULL) + r.d);
-        const uint32_t ncols = min(r.a, W);
         const bool no_gt = r.c != 0;
+        const uint32_t ncols = (BED && no_gt) ? 0u : min(r.a, W);           // .bed: a line without a GT key is all missing
         const int base = (int)((uintptr_t)dst & 15u);
-        const int sh = (int)(((uintptr_t)codes - (uintptr_t)base) & 3u);    // staged byte k of a step holds sample f + k - base
-        for (uint32_t f = 0; f < W; f += DSM_STEP) {
-            const uint32_t n = min(W - f, DSM_STEP);
-            for (uint32_t k = 16u * (uint32_t)lane; k < (uint32_t)base + n; k += 512u) {
-                const int s0 = (int)(f + k) - base;                            // sample of staged byte k
-                const int t0 = s0 - sh;                                        // sample of the aligned word that holds it
-                uint32_t w[5];
-#pragma unroll
-                for (int j = 0; j < 5; ++j) {
-                    const int t = t0 + 4 * j;
-                    w[j] = (!no_gt && t + 3 >= 0 && t < (int)ncols) ? ldw(codes + t) : 0u;
+        // staged byte k of a step holds row byte f + k - base: sample f + k - base (matrix) or 4 (f + k - base) (.bed)
+        const int sh = BED ? (int)((uintptr_t)codes & 3u) : (int)(((uintptr_t)codes - (uintptr_t)base) & 3u);
+        for (uint32_t f = 0; f < R; f += DSM_STEP) {
+            const uint32_t n = min(R - f, DSM_STEP);
+            for (uint32_t k = LB * (uint32_t)lane; k < (uint32_t)base + n; k += 32u * LB) {
+                const int b0 = (int)(f + k) - base;
+                if constexpr (BED) {
+                    const int s0 = 4 * b0;
+                    *reinterpret_cast<uint32_t *>(stage + k) = (s0 >= 0 && s0 + 16 <= (int)ncols) ? ds_bed_lane<false>(codes, s0, sh, ncols, W)
+                                                                                                  : ds_bed_lane<true>(codes, s0, sh, ncols, W);
+                } else {
+                    *reinterpret_cast<uint4 *>(stage + k) = ds_matrix_lane(codes, b0, sh, ncols, no_gt);
                 }
-                uint4 o;
-                o.x = ds_matrix_word(__funnelshift_r(w[0], w[1], 8u * sh), s0, ncols, no_gt);
-                o.y = ds_matrix_word(__funnelshift_r(w[1], w[2], 8u * sh), s0 + 4, ncols, no_gt);
-                o.z = ds_matrix_word(__funnelshift_r(w[2], w[3], 8u * sh), s0 + 8, ncols, no_gt);
-                o.w = ds_matrix_word(__funnelshift_r(w[3], w[4], 8u * sh), s0 + 12, ncols, no_gt);
-                *reinterpret_cast<uint4 *>(stage + k) = o;
             }
             __syncwarp();
             warp_flush_smem(dst + f, stage + base, n, lane);

@@ -282,7 +282,7 @@ class Writer {
 struct Drain {
     std::vector<vcfx_ctx *> ctxs; const RunOptions &opt; Totals &tot; Writer *writer = nullptr; uint64_t line_base = 0;
     long drained = 0, final_index = -1;
-    struct Input { const char *buf; size_t nbytes; size_t tail_out; bool has_data; };
+    struct Input { const char *buf; size_t nbytes; uint64_t file_offset; size_t tail_out; bool has_data; };
     std::deque<Input> inputs;               // the pinned input of every chunk in flight (intact until its slot is acquired again)
     std::string held;                       // hold_trailing_hash: '#' lines waiting for a data line
     int one(std::string &err) {
@@ -290,6 +290,10 @@ struct Drain {
         vcfx_ctx *ctx = ctxs[(size_t)drained % ctxs.size()];        // chunks were dealt round-robin: the oldest one is this context's
         int rc = vcfx_cuda_next_output(ctx, &text, &n, &st);
         if (rc != VCFX_OK) { err = std::string(vcfx_cuda_strerror(rc)) + ": " + vcfx_cuda_last_error(ctx); return rc; }
+        if (opt.on_output && !inputs.empty()) {
+            const Input &in = inputs.front();
+            if (!opt.on_output(in.buf, in.nbytes, in.file_offset, &text, &n)) { err = "output hook failed"; return VCFX_E_INVALID; }
+        }
         if (opt.hold_trailing_hash && !inputs.empty()) {
             const Input &in = inputs.front();
             const size_t tail = std::min(in.tail_out, n);
@@ -341,6 +345,7 @@ int run_stream(Source &src, const RunOptions &opt, Totals &tot, std::string &err
     cfg.chunk_bytes = chunk; cfg.n_slots = 3;
     std::string names_blob; std::vector<uint32_t> name_off;
     if (!opt.query.empty()) { cfg.n_sel = (uint32_t)opt.query.size(); cfg.sel_names = opt.query.data(); }
+    else if (opt.n_sel) cfg.n_sel = opt.n_sel;
     else if (!opt.sel_col.empty()) {
         name_off.push_back(0);
         for (const auto &s : opt.sel_names) { names_blob += s; names_blob.push_back('\t'); name_off.push_back((uint32_t)names_blob.size()); }
@@ -528,7 +533,7 @@ int run_stream(Source &src, const RunOptions &opt, Totals &tot, std::string &err
         rc = vcfx_cuda_submit(ctx, nbytes, &info);
         t_submit += now() - t0;
         {
-            Drain::Input in{buf, nbytes, 0, true};
+            Drain::Input in{buf, nbytes, info.file_offset, 0, true};
             if (opt.hold_trailing_hash) {
                 // the run of '#' and empty lines at the end of the chunk: what it puts out ('#' line + '\n' each), and whether
                 // any data line stands in front of it

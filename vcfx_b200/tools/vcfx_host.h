@@ -76,6 +76,11 @@ struct RunOptions {
     // when set, called once per chunk that has events, in stream order, with the chunk's input bytes and its sorted event
     // list (VCFX_OP_PHASE_CHECK: offset of a dropped line in the chunk << 2 | reason)
     std::function<void(const char *chunk, size_t nbytes, const uint64_t *events, size_t n)> on_events;
+    // when set, called once per drained chunk, in stream order, with the chunk's input bytes, its offset in the whole input
+    // and its output piece, before the piece goes out; it may narrow the piece to what is written (false = stop with an error)
+    std::function<bool(const char *chunk, size_t nbytes, uint64_t file_offset, const char **out, size_t *n)> on_output;
+    // cfg.n_sel for an op that takes a plain count (dosage_calculator's matrix / .bed width W)
+    uint32_t n_sel = 0;
     // genotype_query: the -g argument (cfg.sel_names = its bytes, cfg.n_sel = its length)
     std::string query;
     // nothing is read from the source: the input is `preface` alone
