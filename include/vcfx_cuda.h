@@ -234,6 +234,46 @@ int vcfx_cuda_sync(vcfx_ctx *ctx, vcfx_chunk_stats *stats);
  * and reported (BASELINE.json: any HWE p-value difference must stay within 1e-12 relative and be reported). */
 int vcfx_cuda_hwe_pvalues(int device, const int32_t *counts, size_t n, double *pvalues);
 
+/* ---- pairwise relatedness: KING-robust kinship counts from PLINK 1 .bed rows, on the tensor cores ------------------
+ * An accumulator of its own (no vcfx_cfg, no op).  Each .bed row (VCFX_F_DS_BED's layout: sample s at bits 2 (s & 3) of
+ * byte s >> 2) gives every sample four 0/1 indicators for the variant:
+ *
+ *     code  meaning                                                    plane
+ *     11    hom A2 (REF/REF)                                           A
+ *     10    het                                                        H
+ *     00    hom A1 (ALT/ALT; on a multi-allelic line "any non-REF")    B
+ *     01    missing                                                    none
+ *
+ * and C = A | H | B ("called").  The bits of samples s >= n_samples in a row's last byte are padding and are ignored
+ * whatever their value (a .bed writes 00 there, which would read as hom A1).  Over all rows added, for every ordered pair
+ * (i, j), four uint32 counts:
+ *     CC[i][j]  both called (NSNP)                HH[i][j]  both het (HETHET)
+ *     AB[i][j]  i hom A2 and j hom A1, so IBS0(i, j) = AB[i][j] + AB[j][i]
+ *     HC[i][j]  i het and j called, so HET1 = HC[i][j] and HET2 = HC[j][i]
+ * KING's between-family robust kinship for i < j, in double, is then
+ *     kinship = 0.5 - (HET1 + HET2 - 2 HETHET + 4 IBS0) / (4.0 * min(HET1, HET2))
+ * (the division first, then the subtraction), NA when min(HET1, HET2) = 0.  The numerator is the sum of (x_i - x_j)^2 over
+ * the jointly called sites, so the het counts are restricted to jointly called sites; duplicates give exactly 0.5.
+ * Haploid and multi-allelic calls count as the .bed encodes them.  The counts are integer products (int8 MMAs with s32
+ * accumulation), so they are exact; a run takes at most UINT32_MAX rows in all.
+ * Memory on the device: the four planes (at most about 1 GiB), one slab of rows (vcfx_cuda_king_slab_rows of them) and
+ * 16 x s_pad^2 bytes of counts, s_pad = n_samples rounded up to 256. */
+typedef struct vcfx_king vcfx_king;
+/* no device: VCFX_E_NO_DEVICE; n_samples = 0: VCFX_E_INVALID.  Every copy and kernel runs on `stream`, a cudaStream_t of that
+   device (NULL: the default stream) */
+int  vcfx_cuda_king_create(int device, uint32_t n_samples, void *stream, vcfx_king **out);
+void vcfx_cuda_king_destroy(vcfx_king *k);
+/* n_rows PLINK 1 .bed rows of ceil(n_samples / 4) bytes, back to back.  on_device: a pointer into k's device (enqueued on
+   k's stream) else host memory (may be reused when the call returns).  0 rows is valid.  A call that would take the rows
+   added past UINT32_MAX is refused (VCFX_E_INVALID) and adds nothing.  Rows are gathered into slabs; a full slab is
+   turned into counts on the spot, the rest by vcfx_cuda_king_counts. */
+int  vcfx_cuda_king_add(vcfx_king *k, const void *rows, uint64_t n_rows, int on_device);
+/* waits; writes CC, HH, AB, HC as four row-major n x n uint32 matrices, in that order, to host or device memory
+   (dst_on_device); rows_added (may be NULL) gets the rows added so far.  More rows may be added afterwards. */
+int  vcfx_cuda_king_counts(vcfx_king *k, uint32_t *dst, int dst_on_device, uint64_t *rows_added);
+/* rows of one slab (a multiple of 128): the planes workspace holds this many variants for all samples */
+uint64_t vcfx_cuda_king_slab_rows(const vcfx_king *k);
+
 #ifdef __cplusplus
 }
 #endif

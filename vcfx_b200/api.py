@@ -60,7 +60,8 @@ class ChunkStats(C.Structure):
 EXPORTS = ["vcfx_cuda_abi_version", "vcfx_cuda_device_count", "vcfx_cuda_strerror", "vcfx_cuda_last_error",
            "vcfx_cuda_create", "vcfx_cuda_destroy", "vcfx_cuda_acquire_input", "vcfx_cuda_submit",
            "vcfx_cuda_submit_host", "vcfx_cuda_submit_shared", "vcfx_cuda_set_line_hint", "vcfx_cuda_next_output", "vcfx_cuda_in_flight", "vcfx_cuda_short_lines",
-           "vcfx_cuda_run_device", "vcfx_cuda_sync", "vcfx_cuda_hwe_pvalues"]
+           "vcfx_cuda_run_device", "vcfx_cuda_sync", "vcfx_cuda_hwe_pvalues",
+           "vcfx_cuda_king_create", "vcfx_cuda_king_destroy", "vcfx_cuda_king_add", "vcfx_cuda_king_counts", "vcfx_cuda_king_slab_rows"]
 
 _lib = None
 
@@ -96,6 +97,12 @@ def load():
         l.vcfx_cuda_run_device.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.POINTER(ChunkInfo), C.c_void_p, C.c_size_t]
         l.vcfx_cuda_sync.argtypes = [C.c_void_p, C.POINTER(ChunkStats)]
         l.vcfx_cuda_hwe_pvalues.argtypes = [C.c_int, C.c_void_p, C.c_size_t, C.c_void_p]
+        l.vcfx_cuda_king_create.argtypes = [C.c_int, C.c_uint32, C.c_void_p, C.POINTER(C.c_void_p)]
+        l.vcfx_cuda_king_destroy.argtypes = [C.c_void_p]
+        l.vcfx_cuda_king_add.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_int]
+        l.vcfx_cuda_king_counts.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.POINTER(C.c_uint64)]
+        l.vcfx_cuda_king_slab_rows.argtypes = [C.c_void_p]
+        l.vcfx_cuda_king_slab_rows.restype = C.c_uint64
         _lib = l
     return _lib
 
@@ -756,6 +763,135 @@ def dosage_bed_device(d_in, nbytes: int, mode: int = FILE, width: int | None = N
     views into one output tensor on the same device, written on torch.cuda.current_stream()."""
     names, W, meta, body, tot = _ds_device(d_in, nbytes, mode, width, line_hint, F_DS_BED)
     return DosageBed(names, W, body, *meta, tot, DS_WARNING * tot.short_lines)
+
+
+@dataclass
+class KingCounts:
+    """KING-robust relatedness counts over every ordered pair of samples (include/vcfx_cuda.h, "pairwise relatedness"):
+    cc[i, j] both called, hh[i, j] both het, ab[i, j] i hom A2 (REF/REF) and j hom A1, hc[i, j] i het and j called.
+    int64 tensors [n, n] (CUDA tensors unless counts(device=False) asked for CPU ones)."""
+    cc: object
+    hh: object
+    ab: object
+    hc: object
+    rows: int                      # rows added
+    samples: list | None = None    # the "#CHROM" line's sample names (king() only)
+
+    @property
+    def nsnp(self):
+        return self.cc
+
+    @property
+    def hethet(self):
+        return self.hh
+
+    @property
+    def ibs0(self):
+        return self.ab + self.ab.T
+
+    @property
+    def het1(self):
+        return self.hc
+
+    @property
+    def het2(self):
+        return self.hc.T
+
+    def kinship(self):
+        """KING's between-family robust kinship, float64 [n, n]:
+        0.5 - (HET1 + HET2 - 2 HETHET + 4 IBS0) / (4.0 * min(HET1, HET2)), NaN where min(HET1, HET2) = 0."""
+        import torch
+        het1, het2 = self.het1, self.het2
+        num = (het1 + het2 - 2 * self.hh + 4 * self.ibs0).double()
+        den = torch.minimum(het1, het2)
+        k = 0.5 - num / (4.0 * den.double())
+        return torch.where(den == 0, torch.full_like(k, float("nan")), k)
+
+
+class King:
+    """Accumulator of KING counts (``vcfx_king``) on one GPU.  add() takes PLINK 1 .bed rows — a DosageBed, or a uint8
+    tensor [rows, ceil(n_samples / 4)] on the CPU or on this device — and counts() returns a KingCounts.  The library
+    runs on `stream` (a cudaStream_t handle, 0 = the default stream; None = torch's current stream of the device), so
+    device rows written by torch work on that stream before add() are read after it."""
+
+    def __init__(self, n_samples: int, device: int = 0, stream: int | None = None):
+        self._l = load()
+        self._h = C.c_void_p()
+        self.n_samples, self.device = int(n_samples), int(device)
+        if self.n_samples <= 0:
+            raise ValueError("King needs at least one sample")
+        if stream is None:
+            import torch
+            stream = torch.cuda.current_stream(self.device).cuda_stream
+        rc = self._l.vcfx_cuda_king_create(self.device, self.n_samples, stream or None, C.byref(self._h))
+        if rc != 0:
+            raise VcfxCudaError(rc, self._l.vcfx_cuda_strerror(rc).decode())
+        self.row_bytes = (self.n_samples + 3) // 4
+        self.slab_rows = int(self._l.vcfx_cuda_king_slab_rows(self._h))
+
+    def close(self):
+        if self._h:
+            self._l.vcfx_cuda_king_destroy(self._h)
+            self._h = C.c_void_p()
+
+    def __del__(self):
+        self.close()
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *a):
+        self.close()
+
+    def _add(self, ptr: int, n_rows: int, on_device: bool):
+        rc = self._l.vcfx_cuda_king_add(self._h, ptr, n_rows, int(on_device))
+        if rc != 0:
+            raise VcfxCudaError(rc, self._l.vcfx_cuda_strerror(rc).decode())
+
+    def add(self, x) -> None:
+        import numpy as np
+        import torch
+        if isinstance(x, DosageBed):
+            if x.width != self.n_samples:
+                raise ValueError(f"the rows are {x.width} samples wide, the accumulator has {self.n_samples}")
+            x = x.packed
+        if isinstance(x, np.ndarray):
+            x = torch.from_numpy(x)
+        if x.dtype != torch.uint8 or x.dim() != 2 or x.shape[1] != self.row_bytes:
+            raise ValueError(f"want uint8 rows [n, {self.row_bytes}] for {self.n_samples} samples, got {x.dtype} {tuple(x.shape)}")
+        if x.is_cuda and x.device.index != self.device:
+            raise ValueError(f"the rows are on cuda:{x.device.index}, the accumulator on cuda:{self.device}")
+        x = x.contiguous()
+        self._add(x.data_ptr(), x.shape[0], x.is_cuda)
+
+    def counts(self, device: bool = True) -> KingCounts:
+        """Waits for the rows added so far and returns their counts (int64 tensors on this device, or on the CPU)."""
+        import torch
+        n = self.n_samples
+        rows = C.c_uint64(0)
+        if device:
+            out = torch.empty((4, n, n), dtype=torch.int32, device=f"cuda:{self.device}")
+            rc = self._l.vcfx_cuda_king_counts(self._h, out.data_ptr(), 1, C.byref(rows))
+            big = out.to(torch.int64) & 0xFFFFFFFF
+        else:
+            import numpy as np
+            out = np.empty((4, n, n), dtype=np.uint32)
+            rc = self._l.vcfx_cuda_king_counts(self._h, out.ctypes.data, 0, C.byref(rows))
+            big = torch.from_numpy(out.astype(np.int64))
+        if rc != 0:
+            raise VcfxCudaError(rc, self._l.vcfx_cuda_strerror(rc).decode())
+        return KingCounts(big[0], big[1], big[2], big[3], int(rows.value))
+
+
+def king(data: bytes, mode: int = FILE, width: int | None = None, chunk_bytes: int = 0, **kw) -> KingCounts:
+    """KING counts of a VCF's genotypes: dosage_bed's rows (the streaming path, same rules and errors) into one King on
+    device 0.  Raises ValueError when there are no samples."""
+    bed = dosage_bed(data, mode, width, chunk_bytes, **kw)
+    with King(bed.width) as k:
+        k.add(bed)
+        r = k.counts()
+    r.samples = bed.samples
+    return r
 
 
 F_GQ_STRICT = 1

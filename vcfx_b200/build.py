@@ -27,7 +27,7 @@ ORACLE = ROOT / "oracle"
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 CUDA_LIB = PKG / "libvcfx_cuda.so"
 SYNTH_LIB = PKG / "libvcfx_synth.so"
-TOOL_NAMES = ["allele_freq_calc", "allele_counter", "missing_detector", "variant_counter", "hwe_tester", "nonref_filter", "indexer", "phase_checker", "inbreeding_calculator", "genotype_query", "dosage_calculator", "plink_bed"]
+TOOL_NAMES = ["allele_freq_calc", "allele_counter", "missing_detector", "variant_counter", "hwe_tester", "nonref_filter", "indexer", "phase_checker", "inbreeding_calculator", "genotype_query", "dosage_calculator", "plink_bed", "king"]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

@@ -3,6 +3,7 @@
 // No CPU fallback lives here: without a CUDA device every call fails with VCFX_E_NO_DEVICE.
 #include "vcfx_cuda.h"
 #include "vcfx_kernels.cuh"
+#include "vcfx_king.cuh"
 
 #include <algorithm>
 #include <cctype>
@@ -959,6 +960,138 @@ int vcfx_cuda_hwe_pvalues(int device, const int32_t *counts, size_t n, double *p
         if (cudaGetLastError() != cudaSuccess || cudaMemcpy(pvalues, d_p, n * sizeof(double), cudaMemcpyDeviceToHost) != cudaSuccess) rc = VCFX_E_CUDA;
     }
     cudaFree(d_c); cudaFree(d_p);
+    return rc;
+}
+
+// ---- pairwise relatedness (KING-robust counts): rows are gathered on the device into a slab; a full slab, and the rest at
+// vcfx_cuda_king_counts, becomes the four planes and one MMA launch over every tile
+#ifndef VCFX_KING_PLANES_BYTES
+#ifdef VCFX_EMU
+#define VCFX_KING_PLANES_BYTES ((size_t)1 << 20)      // the emulator's slab borders fall at a few hundred rows, where MMAs are affordable
+#else
+#define VCFX_KING_PLANES_BYTES ((size_t)1 << 30)
+#endif
+#endif
+}  // extern "C"
+
+struct vcfx_king {
+    int device = 0;
+    cudaStream_t stream = nullptr;
+    uint32_t n = 0, s_pad = 0, row_bytes = 0, n_tiles = 0;
+    uint64_t slab_rows = 0, fill = 0, rows_added = 0;
+    size_t plane_stride = 0;
+    uint8_t *d_rows = nullptr, *d_planes = nullptr;
+    uint32_t *d_acc = nullptr, *d_tiles = nullptr;
+};
+
+namespace {
+
+// the planes and one MMA launch for the rows gathered so far
+int king_flush(vcfx_king *k) {
+    if (k->fill == 0) return VCFX_OK;
+    const uint32_t kblocks = (uint32_t)((k->fill + KING_KB - 1) / KING_KB);
+    KingPlanesParams pp = {k->d_rows, k->d_planes, k->plane_stride, (uint32_t)k->fill, k->row_bytes, k->n, k->s_pad};
+    VCFX_LAUNCH(king_planes_kernel, kblocks * (k->s_pad / 128), KING_PLANES_THREADS, 0, k->stream, pp);
+    KingMmaParams mp = {k->d_planes, k->plane_stride, k->d_acc, k->d_tiles, k->s_pad, kblocks};
+    VCFX_LAUNCH(king_mma_kernel, k->n_tiles, KING_MMA_THREADS, KING_MMA_SMEM, k->stream, mp);
+    k->fill = 0;
+    return cudaGetLastError() == cudaSuccess ? VCFX_OK : VCFX_E_CUDA;
+}
+
+}  // namespace
+
+extern "C" {
+
+uint64_t vcfx_cuda_king_slab_rows(const vcfx_king *k) { return k ? k->slab_rows : 0; }
+
+int vcfx_cuda_king_create(int device, uint32_t n_samples, void *stream, vcfx_king **out) {
+    if (!out) return VCFX_E_INVALID;
+    *out = nullptr;
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) return VCFX_E_NO_DEVICE;
+    if (device < 0 || device >= ndev || n_samples == 0) return VCFX_E_INVALID;
+    vcfx_king *k = new (std::nothrow) vcfx_king();
+    if (!k) return VCFX_E_NOMEM;
+    k->device = device;
+    k->n = n_samples;
+    k->s_pad = (uint32_t)(((uint64_t)n_samples + KING_SAMPLE_PAD - 1) / KING_SAMPLE_PAD * KING_SAMPLE_PAD);
+    k->row_bytes = (n_samples + 3) / 4;
+    // the four planes stay within VCFX_KING_PLANES_BYTES (one K block at least)
+    const uint64_t blocks = std::max<uint64_t>(1, VCFX_KING_PLANES_BYTES / (4ull * k->s_pad * KING_KB));
+    k->slab_rows = blocks * KING_KB;
+    k->plane_stride = (size_t)blocks * k->s_pad * KING_KB;
+    // the tiles: every tile of AB and HC, and of CC and HH those that hold an (i, j) with i <= j
+    std::vector<uint32_t> tiles;
+    const uint32_t mt = k->s_pad / KING_TM, nt = k->s_pad / KING_TN;
+    for (uint32_t prob = 0; prob < 4; ++prob)
+        for (uint32_t mi = 0; mi < mt; ++mi)
+            for (uint32_t nj = 0; nj < nt; ++nj)
+                if (prob == KING_AB || prob == KING_HC || (nj + 1) * KING_TN > mi * KING_TM) tiles.push_back(prob << 28 | mi << 14 | nj);
+    k->n_tiles = (uint32_t)tiles.size();
+    auto fail = [&](cudaError_t e) { vcfx_cuda_king_destroy(k); return e == cudaErrorMemoryAllocation ? VCFX_E_NOMEM : VCFX_E_CUDA; };
+    cudaError_t e;
+#define KC(call) do { if ((e = (call)) != cudaSuccess) return fail(e); } while (0)
+    KC(cudaSetDevice(device));
+    k->stream = (cudaStream_t)stream;
+    KC(cudaFuncSetAttribute(king_mma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)KING_MMA_SMEM));
+    KC(cudaMalloc(&k->d_rows, (size_t)k->slab_rows * k->row_bytes));
+    KC(cudaMalloc(&k->d_planes, 4 * k->plane_stride));
+    KC(cudaMalloc(&k->d_acc, 4ull * k->s_pad * k->s_pad * sizeof(uint32_t)));
+    KC(cudaMalloc(&k->d_tiles, tiles.size() * sizeof(uint32_t)));
+    KC(cudaMemcpyAsync(k->d_tiles, tiles.data(), tiles.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, k->stream));
+    KC(cudaMemsetAsync(k->d_acc, 0, 4ull * k->s_pad * k->s_pad * sizeof(uint32_t), k->stream));
+    KC(cudaStreamSynchronize(k->stream));                          // (the tile list is a local vector)
+#undef KC
+    *out = k;
+    return VCFX_OK;
+}
+
+void vcfx_cuda_king_destroy(vcfx_king *k) {
+    if (!k) return;
+    cudaSetDevice(k->device);
+    cudaStreamSynchronize(k->stream);
+    cudaFree(k->d_rows); cudaFree(k->d_planes); cudaFree(k->d_acc); cudaFree(k->d_tiles);
+    delete k;
+}
+
+int vcfx_cuda_king_add(vcfx_king *k, const void *rows, uint64_t n_rows, int on_device) {
+    if (!k || (!rows && n_rows)) return VCFX_E_INVALID;
+    if (n_rows > 0xFFFFFFFFull - k->rows_added) return VCFX_E_INVALID;          // the counts are uint32
+    if (n_rows == 0) return VCFX_OK;
+    if (cudaSetDevice(k->device) != cudaSuccess) return VCFX_E_CUDA;
+    const uint8_t *src = static_cast<const uint8_t *>(rows);
+    for (uint64_t done = 0; done < n_rows;) {
+        const uint64_t take = std::min(n_rows - done, k->slab_rows - k->fill);
+        if (cudaMemcpyAsync(k->d_rows + k->fill * k->row_bytes, src + done * k->row_bytes, take * k->row_bytes,
+                            on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, k->stream) != cudaSuccess)
+            return VCFX_E_CUDA;
+        k->fill += take; done += take; k->rows_added += take;
+        if (k->fill == k->slab_rows) {
+            const int rc = king_flush(k);
+            if (rc != VCFX_OK) return rc;
+        }
+    }
+    // host rows may be reused when this returns (a pinned buffer is read by the copy engine after cudaMemcpyAsync returns)
+    if (!on_device && cudaStreamSynchronize(k->stream) != cudaSuccess) return VCFX_E_CUDA;
+    return VCFX_OK;
+}
+
+int vcfx_cuda_king_counts(vcfx_king *k, uint32_t *dst, int dst_on_device, uint64_t *rows_added) {
+    if (!k || !dst) return VCFX_E_INVALID;
+    if (cudaSetDevice(k->device) != cudaSuccess) return VCFX_E_CUDA;
+    int rc = king_flush(k);
+    if (rc != VCFX_OK) return rc;
+    const size_t bytes = 4ull * k->n * k->n * sizeof(uint32_t);
+    uint32_t *d_dst = dst;
+    if (!dst_on_device && cudaMalloc(&d_dst, bytes) != cudaSuccess) return VCFX_E_NOMEM;
+    KingCountsParams cp = {k->d_acc, d_dst, k->n, k->s_pad};
+    const size_t blocks = std::min<size_t>((bytes / sizeof(uint32_t) + 255) / 256, 148 * 16);
+    VCFX_LAUNCH(king_counts_kernel, (unsigned)blocks, 256, 0, k->stream, cp);
+    if (cudaGetLastError() != cudaSuccess) rc = VCFX_E_CUDA;
+    if (rc == VCFX_OK && !dst_on_device && cudaMemcpyAsync(dst, d_dst, bytes, cudaMemcpyDeviceToHost, k->stream) != cudaSuccess) rc = VCFX_E_CUDA;
+    if (cudaStreamSynchronize(k->stream) != cudaSuccess && rc == VCFX_OK) rc = VCFX_E_CUDA;
+    if (!dst_on_device) cudaFree(d_dst);
+    if (rc == VCFX_OK && rows_added) *rows_added = k->rows_added;
     return rc;
 }
 

@@ -3,7 +3,6 @@
 // (VCFX_OP_DOSAGE + VCFX_F_DS_BED, see include/vcfx_cuda.h).  The host reads the "#CHROM" line for the samples, cuts the
 // .bim fields from each chunk's own bytes at the rows' line offsets, and writes the packed rows behind the .bed magic in
 // file order.  Every file is written under a private name and renamed at the end: a run that fails leaves none behind.
-#include <cctype>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -44,42 +43,6 @@ static const char SHORT_WARNING[] = "Warning: Skipping VCF line with fewer than 
 
 namespace {
 
-// PREFIX.bed / .bim / .fam, each written under a private name until commit()
-struct Outputs {
-    std::string prefix;
-    const char *ext[3] = {".bed", ".bim", ".fam"};
-    int fd[3] = {-1, -1, -1};
-    std::string tmp[3];
-    bool open_all() {
-        for (int i = 0; i < 3; ++i) {
-            tmp[i] = prefix + ext[i] + "." + std::to_string((long)getpid()) + ".part";
-            fd[i] = open(tmp[i].c_str(), O_WRONLY | O_CREAT | O_TRUNC | O_EXCL, 0666);
-            if (fd[i] < 0) { fprintf(stderr, "Error: cannot create '%s%s'\n", prefix.c_str(), ext[i]); return false; }
-        }
-        return true;
-    }
-    void discard() {
-        for (int i = 0; i < 3; ++i) {
-            if (fd[i] >= 0) { close(fd[i]); fd[i] = -1; }
-            if (!tmp[i].empty()) unlink(tmp[i].c_str());
-        }
-    }
-    bool commit() {
-        for (int i = 0; i < 3; ++i) {
-            const int rc = close(fd[i]);
-            fd[i] = -1;
-            if (rc != 0) { fprintf(stderr, "Error: cannot write '%s%s'\n", prefix.c_str(), ext[i]); return false; }
-        }
-        for (int i = 0; i < 3; ++i)
-            if (rename(tmp[i].c_str(), (prefix + ext[i]).c_str()) != 0) {
-                fprintf(stderr, "Error: cannot create '%s%s'\n", prefix.c_str(), ext[i]);
-                for (int j = 0; j < i; ++j) unlink((prefix + ext[j]).c_str());
-                return false;
-            }
-        return true;
-    }
-};
-
 // the first five fields of a tab-separated line (a row's line has ten or more)
 void cut_fields(const char *p, const char *end, const char *f[5], size_t len[5]) {
     for (int i = 0; i < 5; ++i) {
@@ -117,65 +80,16 @@ int main(int argc, char *argv[]) {
         if (fd < 0) { fprintf(stderr, "Error: cannot open file '%s'\n", input); return 1; }
     }
 
-    // ---- up to the first data line: the first "#CHROM" line names the samples (dosage_calculator's file-mode rule)
     vcfxh::Source src(fd);
-    std::string head, chrom;
-    bool found_chrom = false;
-    {
-        std::string buf(1 << 16, '\0');
-        size_t scan = 0;
-        bool eof = false;
-        for (;;) {
-            size_t nl;
-            while ((nl = head.find('\n', scan)) == std::string::npos && !eof) {
-                long r = src.read(&buf[0], buf.size());
-                if (r < 0) { fputs("Error: read error\n", stderr); return 1; }
-                if (r == 0) { eof = true; break; }
-                head.append(buf.data(), (size_t)r);
-            }
-            if (scan >= head.size()) break;
-            size_t end = (nl == std::string::npos) ? head.size() : nl;
-            if (end > scan && head[end - 1] == '\r') --end;
-            if (end > scan) {
-                if (head[scan] != '#') {
-                    if (!found_chrom) { fputs("Error: VCF header (#CHROM) not found before variant records.\n", stderr); return 1; }
-                    break;
-                }
-                if (!found_chrom && end - scan >= 6 && head.compare(scan, 6, "#CHROM") == 0) {
-                    found_chrom = true;
-                    chrom = head.substr(scan, end - scan);
-                }
-            }
-            if (nl == std::string::npos) break;
-            scan = nl + 1;
-        }
-    }
-    if (!found_chrom) { fputs("Error: no #CHROM header line in the input.\n", stderr); return 1; }
+    std::string head;
     std::vector<std::string> names;
-    {
-        size_t p = 0;
-        for (int col = 0;; ++col) {
-            const size_t t = chrom.find('\t', p);
-            const size_t e = t == std::string::npos ? chrom.size() : t;
-            if (col >= 9) names.push_back(chrom.substr(p, e - p));
-            if (t == std::string::npos) break;
-            p = t + 1;
-        }
-        if (!names.empty() && names.back().empty()) names.pop_back();      // an empty column behind a final tab
-    }
-    for (size_t i = 0; i < names.size(); ++i) {
-        bool bad = names[i].empty();
-        for (unsigned char ch : names[i]) bad |= isspace(ch) != 0;
-        if (bad) {
-            fprintf(stderr, "Error: sample %zu ('%s') is empty or contains a blank; .fam is whitespace-delimited.\n", i + 1, names[i].c_str());
-            return 1;
-        }
-    }
+    if (!vcfxh::read_sample_header(src, head, names, ".fam")) return 1;
     const uint32_t W = (uint32_t)names.size();
     const size_t B = ((size_t)W + 3) / 4, row_bytes = 16 + B;
 
-    Outputs outs;
+    vcfxh::AsideFiles outs;
     outs.prefix = prefix;
+    outs.ext = {".bed", ".bim", ".fam"};
     if (!outs.open_all()) { outs.discard(); return 1; }
     std::string fam;
     for (const std::string &n : names) fam += n + "\t" + n + "\t0\t0\t0\t-9\n";

@@ -2,6 +2,7 @@
 #include "vcfx_host.h"
 
 #include <algorithm>
+#include <cctype>
 #include <cerrno>
 #include <cstdlib>
 #include <cstring>
@@ -207,6 +208,94 @@ void finish(int rc) {
     _exit(rc);
 }
 
+bool read_sample_header(Source &src, std::string &head, std::vector<std::string> &names, const char *format) {
+    std::string chrom;
+    bool found_chrom = false;
+    {
+        std::string buf(1 << 16, '\0');
+        size_t scan = 0;
+        bool eof = false;
+        for (;;) {
+            size_t nl;
+            while ((nl = head.find('\n', scan)) == std::string::npos && !eof) {
+                long r = src.read(&buf[0], buf.size());
+                if (r < 0) { fputs("Error: read error\n", stderr); return false; }
+                if (r == 0) { eof = true; break; }
+                head.append(buf.data(), (size_t)r);
+            }
+            if (scan >= head.size()) break;
+            size_t end = (nl == std::string::npos) ? head.size() : nl;
+            if (end > scan && head[end - 1] == '\r') --end;
+            if (end > scan) {
+                if (head[scan] != '#') {
+                    if (!found_chrom) { fputs("Error: VCF header (#CHROM) not found before variant records.\n", stderr); return false; }
+                    break;
+                }
+                if (!found_chrom && end - scan >= 6 && head.compare(scan, 6, "#CHROM") == 0) {
+                    found_chrom = true;
+                    chrom = head.substr(scan, end - scan);
+                }
+            }
+            if (nl == std::string::npos) break;
+            scan = nl + 1;
+        }
+    }
+    if (!found_chrom) { fputs("Error: no #CHROM header line in the input.\n", stderr); return false; }
+    {
+        size_t p = 0;
+        for (int col = 0;; ++col) {
+            const size_t t = chrom.find('\t', p);
+            const size_t e = t == std::string::npos ? chrom.size() : t;
+            if (col >= 9) names.push_back(chrom.substr(p, e - p));
+            if (t == std::string::npos) break;
+            p = t + 1;
+        }
+        if (!names.empty() && names.back().empty()) names.pop_back();      // an empty column behind a final tab
+    }
+    for (size_t i = 0; i < names.size(); ++i) {
+        bool bad = names[i].empty();
+        for (unsigned char ch : names[i]) bad |= isspace(ch) != 0;
+        if (bad) {
+            fprintf(stderr, "Error: sample %zu ('%s') is empty or contains a blank; %s is whitespace-delimited.\n", i + 1, names[i].c_str(), format);
+            return false;
+        }
+    }
+    return true;
+}
+
+bool AsideFiles::open_all() {
+    fd.assign(ext.size(), -1);
+    tmp.assign(ext.size(), std::string());
+    for (size_t i = 0; i < ext.size(); ++i) {
+        tmp[i] = prefix + ext[i] + "." + std::to_string((long)getpid()) + ".part";
+        fd[i] = open(tmp[i].c_str(), O_WRONLY | O_CREAT | O_TRUNC | O_EXCL, 0666);
+        if (fd[i] < 0) { fprintf(stderr, "Error: cannot create '%s%s'\n", prefix.c_str(), ext[i].c_str()); return false; }
+    }
+    return true;
+}
+
+void AsideFiles::discard() {
+    for (size_t i = 0; i < fd.size(); ++i) {
+        if (fd[i] >= 0) { close(fd[i]); fd[i] = -1; }
+        if (!tmp[i].empty()) unlink(tmp[i].c_str());
+    }
+}
+
+bool AsideFiles::commit() {
+    for (size_t i = 0; i < fd.size(); ++i) {
+        const int rc = close(fd[i]);
+        fd[i] = -1;
+        if (rc != 0) { fprintf(stderr, "Error: cannot write '%s%s'\n", prefix.c_str(), ext[i].c_str()); return false; }
+    }
+    for (size_t i = 0; i < fd.size(); ++i)
+        if (rename(tmp[i].c_str(), (prefix + ext[i]).c_str()) != 0) {
+            fprintf(stderr, "Error: cannot create '%s%s'\n", prefix.c_str(), ext[i].c_str());
+            for (size_t j = 0; j < i; ++j) unlink((prefix + ext[j]).c_str());
+            return false;
+        }
+    return true;
+}
+
 int env_device() {
     const char *e = getenv("VCFX_CUDA_DEVICE");
     return e ? atoi(e) : 0;
@@ -392,6 +481,7 @@ int run_stream(Source &src, const RunOptions &opt, Totals &tot, std::string &err
             if (rcs[i] != VCFX_OK) { rc = rcs[i]; err = vcfx_cuda_strerror(rc); destroy_all(); return rc; }
     }
     const size_t G = ctxs.size();
+    if (opt.first_device) *opt.first_device = devices[0];
     double t_create = now() - t_start;
     auto in_flight_total = [&ctxs] { long k = 0; for (vcfx_ctx *c : ctxs) k += vcfx_cuda_in_flight(c); return k; };
 

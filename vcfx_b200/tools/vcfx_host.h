@@ -100,6 +100,9 @@ struct RunOptions {
     std::string preface;
     // a tool that exits right after the run does not tear the CUDA context down (the OS does, faster)
     bool skip_destroy = true;
+    // when set, receives the device of the first context (as the CUDA runtime numbers it once run_stream has narrowed
+    // CUDA_VISIBLE_DEVICES to one GPU) before the first chunk is drained
+    int *first_device = nullptr;
 };
 
 // Streams `src` through libvcfx_cuda. Returns 0, or a negative vcfx_err; err_text gets a message.
@@ -110,5 +113,22 @@ std::vector<int> env_devices();       // VCFX_CUDA_DEVICES=0,1,.. | all (else th
 // flush stdio and leave without running the CUDA runtime's exit handlers (they cost up to a second)
 [[noreturn]] void finish(int rc);
 bool write_all(int fd, const char *p, size_t n);
+
+// The sample names of a VCF for a tool that writes them to a whitespace-delimited file (`format`, e.g. ".fam"), with
+// VCFX_dosage_calculator's file-mode header rule: `src` is read up to the first data line (kept in `head`, which goes back
+// in front of the stream as RunOptions::preface) and the first "#CHROM" line names the samples.  Prints the error and
+// returns false on a read error, a data line before "#CHROM", no "#CHROM" line, or a name that is empty or has a blank.
+bool read_sample_header(Source &src, std::string &head, std::vector<std::string> &names, const char *format);
+
+// Output files PREFIX + ext written under private names and renamed by commit(): a run that fails leaves none behind.
+struct AsideFiles {
+    std::string prefix;
+    std::vector<std::string> ext;
+    std::vector<int> fd;
+    std::vector<std::string> tmp;
+    bool open_all();          // prints the error
+    void discard();
+    bool commit();            // prints the error; on failure the files already renamed are removed again
+};
 
 }  // namespace vcfxh
