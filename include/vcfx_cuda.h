@@ -259,8 +259,9 @@ int vcfx_cuda_hwe_pvalues(int device, const int32_t *counts, size_t n, double *p
  * Memory on the device: the four planes (at most about 1 GiB), one slab of rows (vcfx_cuda_king_slab_rows of them) and
  * 16 x s_pad^2 bytes of counts, s_pad = n_samples rounded up to 256. */
 typedef struct vcfx_king vcfx_king;
-/* no device: VCFX_E_NO_DEVICE; n_samples = 0: VCFX_E_INVALID.  Every copy and kernel runs on `stream`, a cudaStream_t of that
-   device (NULL: the default stream) */
+/* no device: VCFX_E_NO_DEVICE; n_samples = 0 or above 2,097,152 (s_pad past 2^21, the most a tile word indexes):
+   VCFX_E_INVALID, before anything is allocated; counts that do not fit the device: VCFX_E_NOMEM.  Every copy and kernel
+   runs on `stream`, a cudaStream_t of that device (NULL: the default stream) */
 int  vcfx_cuda_king_create(int device, uint32_t n_samples, void *stream, vcfx_king **out);
 void vcfx_cuda_king_destroy(vcfx_king *k);
 /* n_rows PLINK 1 .bed rows of ceil(n_samples / 4) bytes, back to back.  on_device: a pointer into k's device (enqueued on

@@ -811,8 +811,9 @@ class KingCounts:
 class King:
     """Accumulator of KING counts (``vcfx_king``) on one GPU.  add() takes PLINK 1 .bed rows — a DosageBed, or a uint8
     tensor [rows, ceil(n_samples / 4)] on the CPU or on this device — and counts() returns a KingCounts.  The library
-    runs on `stream` (a cudaStream_t handle, 0 = the default stream; None = torch's current stream of the device), so
-    device rows written by torch work on that stream before add() are read after it."""
+    runs on `stream` (a cudaStream_t handle, 0 = the default stream; None = torch's current stream of the device).
+    Device rows given to add() and the tensor counts() writes are ordered after the work queued on torch's current stream
+    at the call, and device rows stay allocated until the library's stream has read them, whichever stream that is."""
 
     def __init__(self, n_samples: int, device: int = 0, stream: int | None = None):
         self._l = load()
@@ -820,9 +821,12 @@ class King:
         self.n_samples, self.device = int(n_samples), int(device)
         if self.n_samples <= 0:
             raise ValueError("King needs at least one sample")
+        if self.n_samples > 0xFFFFFFFF:
+            raise ValueError(f"{self.n_samples} samples do not fit the library's uint32 n_samples")
         if stream is None:
             import torch
             stream = torch.cuda.current_stream(self.device).cuda_stream
+        self._stream = int(stream or 0)
         rc = self._l.vcfx_cuda_king_create(self.device, self.n_samples, stream or None, C.byref(self._h))
         if rc != 0:
             raise VcfxCudaError(rc, self._l.vcfx_cuda_strerror(rc).decode())
@@ -848,6 +852,19 @@ class King:
         if rc != 0:
             raise VcfxCudaError(rc, self._l.vcfx_cuda_strerror(rc).decode())
 
+    def _after_current_stream(self, *used):
+        """The library's stream waits for the work queued so far on torch's current stream (which writes the tensors the
+        library is about to touch), and the caching allocator reuses none of `used` before the library's stream has
+        read it.  Nothing to do when the library runs on the current stream."""
+        import torch
+        cur = torch.cuda.current_stream(self.device)
+        if cur.cuda_stream == self._stream:
+            return
+        mine = torch.cuda.ExternalStream(self._stream, device=self.device) if self._stream else torch.cuda.default_stream(self.device)
+        mine.wait_stream(cur)
+        for t in used:
+            t.record_stream(mine)
+
     def add(self, x) -> None:
         import numpy as np
         import torch
@@ -862,6 +879,8 @@ class King:
         if x.is_cuda and x.device.index != self.device:
             raise ValueError(f"the rows are on cuda:{x.device.index}, the accumulator on cuda:{self.device}")
         x = x.contiguous()
+        if x.is_cuda:
+            self._after_current_stream(x)
         self._add(x.data_ptr(), x.shape[0], x.is_cuda)
 
     def counts(self, device: bool = True) -> KingCounts:
@@ -871,6 +890,7 @@ class King:
         rows = C.c_uint64(0)
         if device:
             out = torch.empty((4, n, n), dtype=torch.int32, device=f"cuda:{self.device}")
+            self._after_current_stream()                # (out is not recorded: the call returns once its stream wrote it)
             rc = self._l.vcfx_cuda_king_counts(self._h, out.data_ptr(), 1, C.byref(rows))
             big = out.to(torch.int64) & 0xFFFFFFFF
         else:

@@ -189,12 +189,19 @@ struct vcfx_ctx {
 
 namespace {
 
+// A runtime failure that becomes a return code is also cleared from the runtime's last error (DESIGN §2): the library
+// links cudart statically, so nobody else clears it, and a later cudaGetLastError() would charge it to a healthy call.
+inline int vcfx_rc(cudaError_t e) {
+    cudaGetLastError();
+    return e == cudaErrorMemoryAllocation ? VCFX_E_NOMEM : VCFX_E_CUDA;
+}
+
 #define CU(call)                                                                         \
     do {                                                                                 \
         cudaError_t _e = (call);                                                         \
         if (_e != cudaSuccess) {                                                         \
             ctx->last_error = std::string(#call) + ": " + cudaGetErrorString(_e);       \
-            return (_e == cudaErrorMemoryAllocation) ? VCFX_E_NOMEM : VCFX_E_CUDA;       \
+            return vcfx_rc(_e);                                                          \
         }                                                                                \
     } while (0)
 
@@ -545,7 +552,7 @@ int vcfx_cuda_create(const vcfx_cfg *cfg, vcfx_ctx **out) {
         cudaError_t _e = (call);                                                         \
         if (_e != cudaSuccess) {                                                         \
             ctx->last_error = std::string(#call) + ": " + cudaGetErrorString(_e);       \
-            return fail(_e == cudaErrorMemoryAllocation ? VCFX_E_NOMEM : VCFX_E_CUDA);   \
+            return fail(vcfx_rc(_e));                                                    \
         }                                                                                \
     } while (0)
     CUC(cudaSetDevice(ctx->device));
@@ -949,18 +956,17 @@ int vcfx_cuda_hwe_pvalues(int device, const int32_t *counts, size_t n, double *p
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) return VCFX_E_NO_DEVICE;
     if (device < 0 || device >= ndev) return VCFX_E_INVALID;
     if (n == 0) return VCFX_OK;
-    if (cudaSetDevice(device) != cudaSuccess) return VCFX_E_CUDA;
+    cudaError_t e = cudaSetDevice(device);
+    if (e != cudaSuccess) return vcfx_rc(e);
     int32_t *d_c = nullptr; double *d_p = nullptr;
-    int rc = VCFX_OK;
-    if (cudaMalloc(&d_c, n * 3 * sizeof(int32_t)) != cudaSuccess || cudaMalloc(&d_p, n * sizeof(double)) != cudaSuccess) rc = VCFX_E_NOMEM;
-    if (rc == VCFX_OK && cudaMemcpy(d_c, counts, n * 3 * sizeof(int32_t), cudaMemcpyHostToDevice) != cudaSuccess) rc = VCFX_E_CUDA;
-    if (rc == VCFX_OK) {
+    if ((e = cudaMalloc(&d_c, n * 3 * sizeof(int32_t))) == cudaSuccess && (e = cudaMalloc(&d_p, n * sizeof(double))) == cudaSuccess &&
+        (e = cudaMemcpy(d_c, counts, n * 3 * sizeof(int32_t), cudaMemcpyHostToDevice)) == cudaSuccess) {
         const int grid = (int)std::min<size_t>((n + 255) / 256, 148 * 8);
         hwe_pvalue_launch(grid, d_c, n, d_p);
-        if (cudaGetLastError() != cudaSuccess || cudaMemcpy(pvalues, d_p, n * sizeof(double), cudaMemcpyDeviceToHost) != cudaSuccess) rc = VCFX_E_CUDA;
+        if ((e = cudaGetLastError()) == cudaSuccess) e = cudaMemcpy(pvalues, d_p, n * sizeof(double), cudaMemcpyDeviceToHost);
     }
     cudaFree(d_c); cudaFree(d_p);
-    return rc;
+    return e == cudaSuccess ? VCFX_OK : vcfx_rc(e);
 }
 
 // ---- pairwise relatedness (KING-robust counts): rows are gathered on the device into a slab; a full slab, and the rest at
@@ -1009,26 +1015,19 @@ int vcfx_cuda_king_create(int device, uint32_t n_samples, void *stream, vcfx_kin
     *out = nullptr;
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) return VCFX_E_NO_DEVICE;
-    if (device < 0 || device >= ndev || n_samples == 0) return VCFX_E_INVALID;
+    const uint64_t s_pad = ((uint64_t)n_samples + KING_SAMPLE_PAD - 1) / KING_SAMPLE_PAD * KING_SAMPLE_PAD;
+    if (device < 0 || device >= ndev || n_samples == 0 || s_pad > KING_MAX_S_PAD) return VCFX_E_INVALID;
     vcfx_king *k = new (std::nothrow) vcfx_king();
     if (!k) return VCFX_E_NOMEM;
     k->device = device;
     k->n = n_samples;
-    k->s_pad = (uint32_t)(((uint64_t)n_samples + KING_SAMPLE_PAD - 1) / KING_SAMPLE_PAD * KING_SAMPLE_PAD);
+    k->s_pad = (uint32_t)s_pad;
     k->row_bytes = (n_samples + 3) / 4;
     // the four planes stay within VCFX_KING_PLANES_BYTES (one K block at least)
     const uint64_t blocks = std::max<uint64_t>(1, VCFX_KING_PLANES_BYTES / (4ull * k->s_pad * KING_KB));
     k->slab_rows = blocks * KING_KB;
     k->plane_stride = (size_t)blocks * k->s_pad * KING_KB;
-    // the tiles: every tile of AB and HC, and of CC and HH those that hold an (i, j) with i <= j
-    std::vector<uint32_t> tiles;
-    const uint32_t mt = k->s_pad / KING_TM, nt = k->s_pad / KING_TN;
-    for (uint32_t prob = 0; prob < 4; ++prob)
-        for (uint32_t mi = 0; mi < mt; ++mi)
-            for (uint32_t nj = 0; nj < nt; ++nj)
-                if (prob == KING_AB || prob == KING_HC || (nj + 1) * KING_TN > mi * KING_TM) tiles.push_back(prob << 28 | mi << 14 | nj);
-    k->n_tiles = (uint32_t)tiles.size();
-    auto fail = [&](cudaError_t e) { vcfx_cuda_king_destroy(k); return e == cudaErrorMemoryAllocation ? VCFX_E_NOMEM : VCFX_E_CUDA; };
+    auto fail = [&](cudaError_t e) { vcfx_cuda_king_destroy(k); return vcfx_rc(e); };
     cudaError_t e;
 #define KC(call) do { if ((e = (call)) != cudaSuccess) return fail(e); } while (0)
     KC(cudaSetDevice(device));
@@ -1037,6 +1036,19 @@ int vcfx_cuda_king_create(int device, uint32_t n_samples, void *stream, vcfx_kin
     KC(cudaMalloc(&k->d_rows, (size_t)k->slab_rows * k->row_bytes));
     KC(cudaMalloc(&k->d_planes, 4 * k->plane_stride));
     KC(cudaMalloc(&k->d_acc, 4ull * k->s_pad * k->s_pad * sizeof(uint32_t)));
+    // the tiles: every tile of AB and HC, and of CC and HH those that hold an (i, j) with i <= j (listed once the counts
+    // have their memory: the list takes at most a 32,768th of it)
+    std::vector<uint32_t> tiles;
+    const uint32_t mt = k->s_pad / KING_TM, nt = k->s_pad / KING_TN;
+    try {
+        for (uint32_t prob = 0; prob < 4; ++prob)
+            for (uint32_t mi = 0; mi < mt; ++mi)
+                for (uint32_t nj = 0; nj < nt; ++nj)
+                    if (prob == KING_AB || prob == KING_HC || (nj + 1) * KING_TN > mi * KING_TM) tiles.push_back(prob << 28 | mi << 14 | nj);
+    } catch (const std::bad_alloc &) {
+        return fail(cudaErrorMemoryAllocation);
+    }
+    k->n_tiles = (uint32_t)tiles.size();
     KC(cudaMalloc(&k->d_tiles, tiles.size() * sizeof(uint32_t)));
     KC(cudaMemcpyAsync(k->d_tiles, tiles.data(), tiles.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, k->stream));
     KC(cudaMemsetAsync(k->d_acc, 0, 4ull * k->s_pad * k->s_pad * sizeof(uint32_t), k->stream));
@@ -1058,13 +1070,14 @@ int vcfx_cuda_king_add(vcfx_king *k, const void *rows, uint64_t n_rows, int on_d
     if (!k || (!rows && n_rows)) return VCFX_E_INVALID;
     if (n_rows > 0xFFFFFFFFull - k->rows_added) return VCFX_E_INVALID;          // the counts are uint32
     if (n_rows == 0) return VCFX_OK;
-    if (cudaSetDevice(k->device) != cudaSuccess) return VCFX_E_CUDA;
+    cudaError_t e = cudaSetDevice(k->device);
+    if (e != cudaSuccess) return vcfx_rc(e);
     const uint8_t *src = static_cast<const uint8_t *>(rows);
     for (uint64_t done = 0; done < n_rows;) {
         const uint64_t take = std::min(n_rows - done, k->slab_rows - k->fill);
-        if (cudaMemcpyAsync(k->d_rows + k->fill * k->row_bytes, src + done * k->row_bytes, take * k->row_bytes,
-                            on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, k->stream) != cudaSuccess)
-            return VCFX_E_CUDA;
+        if ((e = cudaMemcpyAsync(k->d_rows + k->fill * k->row_bytes, src + done * k->row_bytes, take * k->row_bytes,
+                                 on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, k->stream)) != cudaSuccess)
+            return vcfx_rc(e);
         k->fill += take; done += take; k->rows_added += take;
         if (k->fill == k->slab_rows) {
             const int rc = king_flush(k);
@@ -1072,27 +1085,30 @@ int vcfx_cuda_king_add(vcfx_king *k, const void *rows, uint64_t n_rows, int on_d
         }
     }
     // host rows may be reused when this returns (a pinned buffer is read by the copy engine after cudaMemcpyAsync returns)
-    if (!on_device && cudaStreamSynchronize(k->stream) != cudaSuccess) return VCFX_E_CUDA;
+    if (!on_device && (e = cudaStreamSynchronize(k->stream)) != cudaSuccess) return vcfx_rc(e);
     return VCFX_OK;
 }
 
 int vcfx_cuda_king_counts(vcfx_king *k, uint32_t *dst, int dst_on_device, uint64_t *rows_added) {
     if (!k || !dst) return VCFX_E_INVALID;
-    if (cudaSetDevice(k->device) != cudaSuccess) return VCFX_E_CUDA;
+    cudaError_t e = cudaSetDevice(k->device);
+    if (e != cudaSuccess) return vcfx_rc(e);
     int rc = king_flush(k);
     if (rc != VCFX_OK) return rc;
     const size_t bytes = 4ull * k->n * k->n * sizeof(uint32_t);
     uint32_t *d_dst = dst;
-    if (!dst_on_device && cudaMalloc(&d_dst, bytes) != cudaSuccess) return VCFX_E_NOMEM;
+    if (!dst_on_device && (e = cudaMalloc(&d_dst, bytes)) != cudaSuccess) return vcfx_rc(e);
     KingCountsParams cp = {k->d_acc, d_dst, k->n, k->s_pad};
     const size_t blocks = std::min<size_t>((bytes / sizeof(uint32_t) + 255) / 256, 148 * 16);
     VCFX_LAUNCH(king_counts_kernel, (unsigned)blocks, 256, 0, k->stream, cp);
-    if (cudaGetLastError() != cudaSuccess) rc = VCFX_E_CUDA;
-    if (rc == VCFX_OK && !dst_on_device && cudaMemcpyAsync(dst, d_dst, bytes, cudaMemcpyDeviceToHost, k->stream) != cudaSuccess) rc = VCFX_E_CUDA;
-    if (cudaStreamSynchronize(k->stream) != cudaSuccess && rc == VCFX_OK) rc = VCFX_E_CUDA;
+    e = cudaGetLastError();
+    if (e == cudaSuccess && !dst_on_device) e = cudaMemcpyAsync(dst, d_dst, bytes, cudaMemcpyDeviceToHost, k->stream);
+    const cudaError_t es = cudaStreamSynchronize(k->stream);
+    if (e == cudaSuccess) e = es;
     if (!dst_on_device) cudaFree(d_dst);
-    if (rc == VCFX_OK && rows_added) *rows_added = k->rows_added;
-    return rc;
+    if (e != cudaSuccess) return vcfx_rc(e);
+    if (rows_added) *rows_added = k->rows_added;
+    return VCFX_OK;
 }
 
 }  // extern "C"

@@ -24,6 +24,7 @@ constexpr uint32_t KING_STAGES = 4;
 constexpr uint32_t KING_A_BYTES = KING_TM * KING_KB, KING_B_BYTES = KING_TN * KING_KB;
 constexpr uint32_t KING_STAGE_BYTES = KING_A_BYTES + KING_B_BYTES;
 constexpr uint32_t KING_SAMPLE_PAD = KING_TN;           // samples are padded to a multiple of both tile sides
+constexpr uint64_t KING_MAX_S_PAD = (uint64_t)KING_TM << 14;   // a tile word holds the tile row in 14 bits: 2,097,152 samples
 constexpr uint32_t KING_MMA_THREADS = 192;              // warp 0 loads, warp 1 issues the MMAs, warps 2-5 drain the tile
 constexpr uint32_t KING_PLANES_THREADS = 256;
 // 1024 bytes to align the ring to the swizzle atom, the ring, then 2 x STAGES + 1 mbarriers and the TMEM address
